@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: generated frames/sec end-to-end (100-step DiT + VAE decode), BASELINE.json.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c1|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c1|c5] [--dump-outputs DIR]
 
 A *step* is one complete rollout batch of the README inference shape (BASELINE config 2: B=1 rollout,
 32 frames, 4 prompt frames, 100 noise steps => 28 generated frames x 101 DiT evaluations, plus VAE
@@ -21,6 +21,8 @@ kernels).  One JSON line is printed by rank 0:
            torch eager on this GPU (informational)
 With --impl reference only the CPU arm runs (the Python reference cannot travel to the GPU box; the
 oracle port is its restatement) and prints the same line with "impl": "reference".
+--dump-outputs DIR writes what the last timed step returned (dump_outputs); the inputs depend only on the arguments, so
+two builds run with the same arguments can be compared file by file.
 N > 1 (torchrun): every rank runs its own rollouts (weak scaling, no collective on the data path); every collective
 of this file is in barrier() / timed(), called the same number of times by every rank.
 """
@@ -56,6 +58,7 @@ WORKLOADS = {
 DIT_STEP_GFLOP = 589.09          # per sample, 5-frame window (SURVEY.md section 8(d))
 DIT_GEMM_GFLOP = 579.8           # the four per-half GEMMs only
 VAE_ENC_GFLOP, VAE_DEC_GFLOP = 96.58, 191.69
+DUMP_MAX_ELEMS = 15_000_000      # float32 values over all --dump-outputs files: 60 MB, under 64 MB with the .npy headers
 
 
 def peaks():
@@ -110,6 +113,21 @@ class ClockSampler:
         # "under load": upper half of the samples (the loop is busy the whole time; idle tails drop out)
         med = sm[len(sm) * 3 // 4] if sm else None
         return dict(sm_mhz=med, sm_max_mhz=smax, reasons=sorted(reasons), samples=len(sm))
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy in float32 (uint8 frames convert exactly).  An array larger than its share
+    of DUMP_MAX_ELEMS is written as a fixed sample instead: a flat vector of its elements at sorted indices drawn from a
+    CPU generator seeded with 0, so the same shape always gives the same indices."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_MAX_ELEMS // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > share:
+            idx = torch.randint(t.numel(), (share,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------ product arm
@@ -338,16 +356,18 @@ def bench_config(wl, B):
 def run_reference_arm(args, wl, rank, world):
     """The reference's own CPU implementation of the path (oracle port: the Python reference cannot travel to the GPU
     box) on all host cores.  One step = one bounded sample = BASELINE config 1 in full (the same code path with 44
-    instead of 2,828 DiT steps).  As many of the requested warm-up + timed steps are run as fit ~4 minutes (at least
-    one warm-up and one timed sample); `samples_run` says how many."""
+    instead of 2,828 DiT steps); --warmup untimed samples, then --steps timed ones."""
     if rank != 0:
         return
     t_all = time.perf_counter()
-    want = args.warmup + args.steps
-    first = cpu_baseline(wl)                                        # warm-up sample (pages in torch / MKL, builds the weights)
-    per = time.perf_counter() - t_all
-    n_timed = max(1, min(args.steps, int((240.0 - per) / max(per, 1e-3))))
-    vals = [cpu_baseline(wl) for _ in range(n_timed)]
+    for _ in range(args.warmup):                                    # pages in torch / MKL
+        cpu_c1_run()
+    vals = []
+    for _ in range(args.steps):
+        c1 = cpu_c1_run()
+        vals.append(cpu_baseline(wl, c1))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(latents=c1["latents"], frames=c1["frames"]))
     v = sum(c["value"] for c in vals) / len(vals)
     cb = dict(vals[-1], value=round(v, 6))
     gen = wl["total"] - wl["n_prompt"]
@@ -357,7 +377,7 @@ def run_reference_arm(args, wl, rank, world):
                 data="synthetic", config=bench_config(wl, wl["B"]),
                 algorithm="dense (every step recomputes the whole 5-frame window): the reference's own schedule, CPU fp32",
                 cpu_baseline=cb, e2e=dict(value=cb["value"], unit=UNIT, h2d_bytes_per_step=0, d2h_bytes_per_step=0),
-                gpu_launches=0, samples_run=dict(requested=want, warmup=1, timed=n_timed, first_sample_value=first["value"]),
+                gpu_launches=0, samples_run=dict(warmup=args.warmup, timed=args.steps),
                 extrapolated_ms_per_rollout=round(1000.0 * gen / v, 1),
                 note="ms_per_step is the wall time of one bounded sample (config 1 in full: 44 DiT steps + 4 encodes + 8 decodes); "
                      "value scales its measured per-step times to the workload's step count",
@@ -469,7 +489,13 @@ def main():
     ap.add_argument("--no-c3", action="store_true", help="skip the B=8 legs (BASELINE config 3 and the dense window step at B=8)")
     ap.add_argument("--no-c1", action="store_true", help="skip the product run of BASELINE config 1")
     ap.add_argument("--no-eager", action="store_true", help="skip the torch-eager-on-GPU informational baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (fp32 latents, uint8 frames; rank 0's "
+                         "rollouts) as DIR/<name>.npy in float32, at most 60 MB: a larger array becomes a fixed seeded sample of "
+                         "its elements")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     wl = dict(WORKLOADS[args.workload])
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -517,8 +543,11 @@ def main():
     gens = rollout_generators(my_ids, dev)
     out_host = torch.empty((B, total, 360, 640, 3), dtype=torch.uint8).pin_memory()
 
+    last = {}                                    # what the latest resident step returned, for --dump-outputs
+
     def rollout_resident():
-        frames, _ = sampler.generate(prompt_dev, actions, total, generator=gens)
+        frames, lat = sampler.generate(prompt_dev, actions, total, generator=gens)
+        last.update(latents=lat, frames=frames)
         return frames
 
     def rollout_e2e():
@@ -552,6 +581,9 @@ def main():
     with ClockSampler(local) as cs:
         ms_total = timed(rollout_resident, args.steps)
     clocks = cs.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
     rollout_e2e()
     ms_e2e = timed(rollout_e2e, args.steps)
 
