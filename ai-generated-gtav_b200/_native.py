@@ -13,7 +13,8 @@ LIB_PATH = os.path.join(_HERE, "libgtav_b200.so")
 
 # every symbol include/gtav_b200.h declares (tests check the .so exports exactly these)
 EXPORTS = [
-    "gtav_last_error", "gtav_abi_version", "gtav_gemm_bf16", "gtav_gemm_skinny_bf16", "gtav_gemm_skinny_tagged_bf16", "gtav_gemm_skinny_workspace_bytes",
+    "gtav_last_error", "gtav_abi_version", "gtav_gemm_bf16", "gtav_gemm_skinny_bf16", "gtav_gemm_skinny_tagged_bf16", "gtav_gemm_skinny_fused_bf16",
+    "gtav_gemm_skinny_workspace_bytes",
     "gtav_dit_context", "gtav_dit_last_frame", "gtav_attention_temporal_last", "gtav_ln_modulate", "gtav_ln_affine",
     "gtav_attention_seq", "gtav_attention_temporal", "gtav_ddim_update", "gtav_dit_create", "gtav_dit_destroy",
     "gtav_dit_mod_width", "gtav_dit_workspace_bytes", "gtav_dit_plan_create", "gtav_dit_plan_destroy",
@@ -81,6 +82,8 @@ def load() -> C.CDLL:
         "gtav_gemm_bf16": [vp, i, vp, i, vp, i, i, i, i, i, vp, vp, i, vp, i, ip, i, i, vp],
         "gtav_gemm_skinny_bf16": [vp, i, vp, i, vp, i, i, i, i, i, vp, vp, i, vp, i, ip, i, i, vp, vp, vp],
         "gtav_gemm_skinny_tagged_bf16": [vp, i, vp, i, vp, i, i, i, i, i, vp, vp, i, vp, i, ip, i, i, vp, i, vp],
+        "gtav_gemm_skinny_fused_bf16": [vp, i, vp, i, vp, i, i, i, i, vp, vp, i, vp, i, ip, i, vp, ip, i, vp, vp, i, i, i, vp, fp,
+                                        i, i, i, vp],
         "gtav_dit_context": [vp, vp, i, ip, vp],
         "gtav_dit_last_frame": [vp, vp, i, ip, vp, vp],
         "gtav_ln_modulate": [vp, vp, i, i, vp, i, i, i, ip, i, vp],

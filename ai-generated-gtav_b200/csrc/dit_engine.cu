@@ -282,7 +282,7 @@ int run_backbone(gtav_dit_plan_s* p, const Shape* sh, int mode, const void* x, i
 extern "C" {
 
 const char* gtav_last_error(void) { return get_error(); }
-int gtav_abi_version(void) { return 4; }
+int gtav_abi_version(void) { return 5; }
 
 int gtav_dit_create(const gtav_dit_config* cfg, const gtav_dit_weights* w, gtav_dit_t* out) {
     if (!cfg || !w || !out) { set_error("dit_create: null argument"); return -1; }
@@ -440,7 +440,8 @@ size_t gtav_gemm_skinny_workspace_bytes(int M) { return skinny_workspace_bytes(M
 namespace {
 int skinny_standalone(const void* A, int lda, const void* W, int ldw, void* out, int ldo, int M, int N, int K, int epilogue,
                       const void* bias, const void* res, int ldr, const void* gate, int gate_ld, const int* frame_row,
-                      int rows_per_frame, int splits, void* workspace, int* counters, int tag, gtav_stream_t stream) {
+                      int rows_per_frame, int splits, void* workspace, int* counters, int tag, gtav_stream_t stream,
+                      const SkinnyFuseParams* fuse = nullptr) {
     GemmParams p{};
     p.out = static_cast<bf16*>(out); p.ldo = ldo; p.bias = static_cast<const bf16*>(bias);
     p.res = static_cast<const bf16*>(res); p.ldr = ldr; p.gate = static_cast<const bf16*>(gate); p.gate_ld = gate_ld;
@@ -448,7 +449,7 @@ int skinny_standalone(const void* A, int lda, const void* W, int ldw, void* out,
     p.M = M; p.N = N; p.K = K;
     SkinnyOp op;
     int rc = skinny_prepare(&op, static_cast<const bf16*>(A), lda, static_cast<const bf16*>(W), ldw, p, epilogue,
-                            static_cast<float*>(workspace), counters, splits);
+                            static_cast<float*>(workspace), counters, splits, fuse);
     if (rc) return rc;
     op.tag = tag;
     if (const char* t = getenv("GTAV_SKINNY_TRACE")) op.trace = reinterpret_cast<long long*>(strtoull(t, nullptr, 0));
@@ -473,6 +474,29 @@ int gtav_gemm_skinny_tagged_bf16(const void* A, int lda, const void* W, int ldw,
     if (parity != 0 && parity != 1) { set_error("gemm_skinny_tagged: parity must be 0 or 1, got %d", parity); return -1; }
     return skinny_standalone(A, lda, W, ldw, out, ldo, M, N, K, epilogue, bias, res, ldr, gate, gate_ld, frame_row, rows_per_frame,
                              splits, workspace, nullptr, 2 | parity, stream);
+}
+
+int gtav_gemm_skinny_fused_bf16(const void* A, int lda, const void* W, int ldw, void* out, int ldo, int M, int N, int K,
+                                const void* bias, const void* res, int ldr, const void* gate, int gate_ld, const int* frame_row,
+                                int splits, void* workspace, int* counters, int mode, void* ln_out, const void* ln_mod,
+                                int ln_mod_ld, int ln_shift_off, int ln_scale_off, const void* kv_cache, const float* rot,
+                                int ctx_frames, int positions, int parity, gtav_stream_t stream) {
+    if (!workspace) { set_error("gemm_skinny_fused: workspace is required"); return -1; }
+    if (parity < -1 || parity > 1) { set_error("gemm_skinny_fused: parity must be -1, 0 or 1, got %d", parity); return -1; }
+    if (parity == -1 && !counters) { set_error("gemm_skinny_fused: counters are required with parity -1"); return -1; }
+    if (mode != SK_FUSE_LN && mode != SK_FUSE_TATTN) { set_error("gemm_skinny_fused: mode must be 1 or 2, got %d", mode); return -1; }
+    SkinnyFuseParams f{};
+    f.mode = mode;
+    f.ln_out = static_cast<bf16*>(ln_out);
+    f.ln_mod = static_cast<const bf16*>(ln_mod);
+    f.ln_mod_ld = ln_mod_ld; f.ln_shift_off = ln_shift_off; f.ln_scale_off = ln_scale_off;
+    f.kv_cache = static_cast<const bf16*>(kv_cache);
+    f.rot = reinterpret_cast<const float2*>(rot);
+    f.ctx_frames = ctx_frames; f.positions = positions;
+    // the mode fixes the epilogue (skinny_prepare checks every other argument against it)
+    const int epi = mode == SK_FUSE_LN ? EPI_BIAS_GATE_RES : EPI_STORE;
+    return skinny_standalone(A, lda, W, ldw, out, ldo, M, N, K, epi, bias, res, ldr, gate, gate_ld, frame_row, 144, splits,
+                             workspace, parity == -1 ? counters : nullptr, parity == -1 ? 0 : 2 | parity, stream, &f);
 }
 
 int gtav_ln_modulate(const void* x, void* out, int M, int D, const void* mod, int mod_ld, int shift_off, int scale_off,

@@ -32,7 +32,8 @@ extern "C" {
 typedef struct CUstream_st* gtav_stream_t; /* == cudaStream_t */
 
 const char* gtav_last_error(void);
-/* ABI version; bumped on any signature change or new entry point (4: gtav_gemm_skinny_tagged_bf16, larger DiT plan workspace). */
+/* ABI version; bumped on any signature change or new entry point (4: gtav_gemm_skinny_tagged_bf16, larger DiT plan workspace;
+ * 5: gtav_gemm_skinny_fused_bf16). */
 int gtav_abi_version(void);
 
 /* ------------------------------------------------------------------------------------------
@@ -78,6 +79,22 @@ int gtav_gemm_skinny_tagged_bf16(const void* A, int lda, const void* W, int ldw,
                                  int epilogue, const void* bias, const void* res, int ldr, const void* gate, int gate_ld,
                                  const int* frame_row, int rows_per_frame, int splits, void* workspace, int parity,
                                  gtav_stream_t stream);
+/* The same GEMM with the row-wise kernel that follows it in a last-frame DiT pass folded into its split-K reduce, as the
+ * engine runs to_out / fc2 and the temporal to_qkv.  The mode fixes the epilogue:
+ *   mode 1 (LayerNorm): N = 1024, 4, 8 or 16 splits, epilogue BIAS_GATE_RES with 144 rows per frame (res may be out).  out
+ *          receives the new residual stream; ln_out [M, 1024] (contiguous) receives gtav_ln_modulate of those rows with shift /
+ *          scale at ln_mod + frame * ln_mod_ld + {ln_shift_off, ln_scale_off}, frame from frame_row as for the gate;
+ *   mode 2 (temporal attention): N = 3072 (q | k | v of 16 heads), 4 splits, epilogue STORE.  out [M, 1024] receives
+ *          gtav_attention_temporal_last of the q|k|v rows (B = M / positions) against kv_cache with ctx_frames (0..7) cached
+ *          frames and rot [ctx_frames + 1][32] (cos, sin); the q|k|v rows themselves are not stored.
+ * Both give the bits of the unfused launch followed by gtav_ln_modulate / gtav_attention_temporal_last.  parity -1: the CTAs
+ * meet on `counters` (as gtav_gemm_skinny_bf16); 0 or 1: tagged exchange under the protocol of gtav_gemm_skinny_tagged_bf16
+ * (counters unused).  All CTAs of a launch (one per token row, up to the SM count) must be co-resident. */
+int gtav_gemm_skinny_fused_bf16(const void* A, int lda, const void* W, int ldw, void* out, int ldo, int M, int N, int K,
+                                const void* bias, const void* res, int ldr, const void* gate, int gate_ld, const int* frame_row,
+                                int splits, void* workspace, int* counters, int mode, void* ln_out, const void* ln_mod,
+                                int ln_mod_ld, int ln_shift_off, int ln_scale_off, const void* kv_cache, const float* rot,
+                                int ctx_frames, int positions, int parity, gtav_stream_t stream);
 
 /* modulate(LayerNorm(x), shift, scale) of dit.py:19-27 -> bf16 [M, D]; D = 1024. */
 int gtav_ln_modulate(const void* x, void* out, int M, int D, const void* mod, int mod_ld, int shift_off, int scale_off,

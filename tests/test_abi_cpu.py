@@ -33,7 +33,7 @@ def test_library_exports_exactly_the_header(native):
     out = subprocess.run(["nm", "-D", "--defined-only", native.LIB_PATH], capture_output=True, text=True).stdout
     exported = sorted(l.split()[-1] for l in out.splitlines() if " T " in l)
     assert exported == decl, set(exported) ^ set(decl)          # nothing else leaks out of the .so
-    assert lib.gtav_abi_version() == 4
+    assert lib.gtav_abi_version() == 5
 
 
 def test_library_is_sm100a_tcgen05(native):
@@ -57,6 +57,20 @@ def test_host_side_argument_checks_need_no_gpu(native):
     assert lib.gtav_gemm_skinny_tagged_bf16(*args, None, 1, None) != 0 and b"workspace" in lib.gtav_last_error()
     assert lib.gtav_gemm_skinny_tagged_bf16(*args, 4096, 2, None) != 0 and b"parity" in lib.gtav_last_error()
     assert lib.gtav_gemm_skinny_workspace_bytes(144) == 160 * 144 * 128 * 4
+    # the fused-reduce entry point: the same host checks, then skinny_prepare's refusals of a shape the fused mode cannot
+    # run, all before any descriptor or launch (the non-null device addresses below are never dereferenced)
+    fake = 4096
+
+    def fused(mode, N, ws=fake, counters=None, ctx_frames=0, parity=0):
+        return lib.gtav_gemm_skinny_fused_bf16(fake, 1024, fake, 1024, fake, N, 144, N, 1024, fake, fake, N, fake, N, None, 4, ws,
+                                               counters, mode, fake, fake, 6 * 1024, 0, 1024, fake, fake, ctx_frames, 144, parity,
+                                               None)
+    assert fused(1, 1024, ws=None) != 0 and b"workspace" in lib.gtav_last_error()
+    assert fused(1, 1024, parity=2) != 0 and b"parity" in lib.gtav_last_error()
+    assert fused(1, 1024, parity=-1) != 0 and b"counters" in lib.gtav_last_error()
+    assert fused(0, 1024) != 0 and b"mode" in lib.gtav_last_error()
+    assert fused(1, 2048) != 0 and b"fused reduce mode 1 does not fit" in lib.gtav_last_error()      # LayerNorm: N = 1024 only
+    assert fused(2, 3072, ctx_frames=8) != 0 and b"fused reduce mode 2 does not fit" in lib.gtav_last_error()   # <= 7 cached frames
 
 
 def test_dit_state_dict_contract():

@@ -425,8 +425,7 @@ def test_temporal_attention_last_frame_matches_dense(lib):
     N.check(fn(last_qkv.data_ptr(), out.data_ptr(), B, T - 1, P, H, rot.data_ptr(), cache.data_ptr(), N.current_stream()), "last")
     torch.cuda.synchronize()
     ref = dense.view(B, T, P, D)[:, T - 1].reshape(B * P, D)
-    err = float((out.float() - ref.float()).abs().max())
-    assert err <= 2 ** -7 * float(ref.float().abs().max()), err
+    assert torch.equal(out, ref), float((out.float() - ref.float()).abs().max())
 
 
 
