@@ -174,6 +174,7 @@ struct AttnCfg {
     static_assert(SEQ % KB == 0 && KB % 16 == 0 && KB <= 256 && (KB % 32 == 0 || KB % 32 == 16), "key blocking");
     static_assert((KB * AT_ROWB) % 1024 == 0, "key blocks must start on a swizzle-atom boundary");
     static_assert(NBUF >= 1 && NBUF <= 4 && TM_O + 64 * OBUF <= TMC && (TMC == 256 || TMC == 512), "TMEM budget");
+    static_assert(G >= NBUF, "the S_FULL wait of the softmax groups assumes no more S buffers than groups");
     static_assert(SMEM <= 232448, "shared memory budget");
 };
 
@@ -341,15 +342,10 @@ attn_tc_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int heads, 
             const uint32_t k = n % NBUF, u = n / NBUF;                   // S buffer and how often it has been used before
             // A parity wait only tells the current phase from the previous one, so before waiting for phase u of S_FULL[k] the
             // group must know that phase u - 1 (the buffer's previous use, block n - NBUF) has completed.
-            //  * G < NBUF: it does - the group's own previous block n - G came later in the tensor pipe's in-order sequence
-            //    than block n - NBUF, and the group has consumed it.  (An explicit wait for phase u - 1 would be WRONG here:
-            //    S(n) may already be complete - the other groups run ahead through the spare buffers - and a wait for parity
-            //    u - 1 = parity u + 1 then blocks on the phase this very group has to enable: the scheduler stall of the
-            //    144-key / 3-buffer / 2-group form.)
             //  * NBUF a multiple of G: the previous use was this group's own block.
             //  * otherwise (NBUF = 1, G = 2: two blocks in all): go through phase u - 1 first; S(n) cannot be complete yet,
             //    it needs the P V product of block n - NBUF >= n - G + 1, i.e. of a block not older than this group's last.
-            if (G >= NBUF && (NBUF % G) != 0 && u > 0) mbar_wait(&bars[B_SFULL + k], (u - 1) & 1);
+            if ((NBUF % G) != 0 && u > 0) mbar_wait(&bars[B_SFULL + k], (u - 1) & 1);
             mbar_wait(&bars[B_SFULL + k], u & 1);
             tcgen05_fence_after();
             if (tr) AT_STAMP(tr_role);                                   // S full
@@ -395,22 +391,14 @@ attn_tc_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int heads, 
             // a group of G >= 3 skipped two phases between its waits, and a parity wait posted while the barrier was still
             // two phases behind returned at once: stale maximum, arrivals in the wrong phase and, eventually, a stalled
             // scheduler (seen once in a VAE decode, never in the unit tests).
-#ifdef GTAV_ATTN_SINGLE_MREADY                         // the former single-barrier chain, kept to show that the stress test catches it
-            if (n > 0) mbar_wait(&bars[B_MREADY], (n - 1) & 1);
-#else
             if (n > 0) mbar_wait(&bars[B_MREADY + (n - 1) % G], ((n - 1) / G) & 1);
-#endif
             if (j > 0) {
                 const float m_prev = sM[row];
                 if ((bm - m_prev) * sl2 > AT_LAZY) o_scale = ex2_approx((m_prev - bm) * sl2);
                 else m_use = m_prev;
             }
             sM[row] = m_use;
-#ifdef GTAV_ATTN_SINGLE_MREADY
-            mbar_arrive(&bars[B_MREADY]);
-#else
             mbar_arrive(&bars[B_MREADY + n % G]);
-#endif
             if (tr) AT_STAMP(tr_role);                                   // row maximum handed on
             if (j < G) {                                                 // this group's first block of the tile (its blocks are G apart)
                 l = 0.f;
@@ -647,19 +635,13 @@ int launch_attention_tc(const bf16* qkv, bf16* out, int groups, int seq, int hea
                         cudaStream_t s) {
     if (groups <= 0) return 0;
     if (seq == 576 && rot_pairs == 16) {
-        // Default: 4 key blocks of 144 keys per query tile in THREE S buffers, one softmax warpgroup per buffer (480 threads):
-        // a group's next S tile is computed while it works on the current one, instead of waiting for its own P V product to
+        // 4 key blocks of 144 keys per query tile in THREE S buffers, one softmax warpgroup per buffer (480 threads): a
+        // group's next S tile is computed while it works on the current one, instead of waiting for its own P V product to
         // release one of two buffers.  32 frames: 122.8 us against 131.8 us for 3 blocks of 192 keys in 2 buffers with 2
-        // groups (GTAV_ATTN_KB=192); 6 blocks of 96 keys in 4 buffers: 146 us with 2 groups (GTAV_ATTN_KB=96), 146 us with 4
-        // (964) - the per-block hand-offs cost more than the extra buffers save.  144 keys x 3 buffers with TWO groups
-        // (GTAV_ATTN_KB=1442; a spare buffer per group, so no group ever waits for its own P V product): 132 us - the third
-        // buffer alone buys nothing, the third group's instruction issue does.
-        const char* e = getenv("GTAV_ATTN_KB");
-        const int kb = e != nullptr ? atoi(e) : 0;
-        if (kb == 96) return launch_tc<576, 96, 4, 512, 2, 16>(qkv, out, groups, heads, rot, s);
-        if (kb == 964) return launch_tc<576, 96, 4, 512, 4, 16>(qkv, out, groups, heads, rot, s);
-        if (kb == 192) return launch_tc<576, 192, 2, 512, 2, 16>(qkv, out, groups, heads, rot, s);
-        if (kb == 1442) return launch_tc<576, 144, 3, 512, 2, 16>(qkv, out, groups, heads, rot, s);
+        // groups; 6 blocks of 96 keys in 4 buffers: 146 us with 2 groups, 146 us with 4 - the per-block hand-offs cost more
+        // than the extra buffers save.  144 keys x 3 buffers with TWO groups (a spare buffer per group, so no group ever
+        // waits for its own P V product): 132 us - the third buffer alone buys nothing, the third group's instruction issue
+        // does.
         return launch_tc<576, 144, 3, 512, 3, 16>(qkv, out, groups, heads, rot, s);
     }
     // S = 144: one S buffer and one O buffer in 256 TMEM columns, 72 KB of shared memory -> two CTAs per SM hide each other's

@@ -2,7 +2,6 @@
 // enqueues the kernel sequence that stands in for DiT.forward (reference model/dit.py:343-376) and
 // SpatioTemporalDiTBlock.forward (model/dit.py:200-225).  No allocation, no host sync: everything is
 // launched on the caller's stream so a whole step can be captured into a CUDA graph.
-#include <stdio.h>
 #include <stdlib.h>
 
 #include <new>
@@ -139,11 +138,8 @@ int build_shape(gtav_dit_plan_s* p, Shape* sh, int frames, bool allow_skinny) {
     if (sh->sk[1]) sh->s_out.resize(nh);
     if (sh->sk[2]) sh->s_fc1.resize(nh);
     if (sh->sk[3]) sh->s_fc2.resize(nh);
-    // GTAV_SK_SPLITS="qkv,out,fc1,fc2": K-split override per GEMM kind (0 = the library's choice), for A/B measurements
-    int so[4] = {0, 0, 0, 0};
-    if (const char* e = getenv("GTAV_SK_SPLITS")) sscanf(e, "%d,%d,%d,%d", &so[0], &so[1], &so[2], &so[3]);
     sh->fuse_ln = sh->sk[1] && sh->sk[3] && fuse_enabled();
-    sh->fuse_tattn = sh->sk[0] && fuse_enabled() && (so[0] > 0 ? so[0] : skinny_pick_splits(M, 3 * D, D)) == 4 && p->T - 1 <= 7;
+    sh->fuse_tattn = sh->sk[0] && fuse_enabled() && skinny_pick_splits(M, 3 * D, D) == 4 && p->T - 1 <= 7;
     const size_t cache_layer = static_cast<size_t>(p->B) * (p->T - 1) * S * 2 * D;
     for (int i = 0; i < nh && rc == 0; ++i) {
         const gtav_dit_half& hw = h->halves[i];
@@ -158,16 +154,12 @@ int build_shape(gtav_dit_plan_s* p, Shape* sh, int frames, bool allow_skinny) {
         // weight-streaming kernel: measured in the real step (scripts/bench_graph.py --engine), a prefetch issued at its
         // start competes with its own slab loads (1.208 vs 1.191 ms per step, round 1), and one issued after its MMAs -
         // when HBM is idle - still costs 2 % (1.191 vs 1.169 ms, round 2): the next launch's slab request is not what its
-        // critical path waits for.  GTAV_PREFETCH=0 / 1 forces off / on everywhere.
+        // critical path waits for.
         const size_t DD = static_cast<size_t>(D) * D * 2;
-        const char* pfenv = getenv("GTAV_PREFETCH");
-        const bool pf_off = pfenv != nullptr && pfenv[0] == '0', pf_force = pfenv != nullptr && pfenv[0] == '1';
-        if (!pf_off) {
-            if (pf_force || !sh->sk[0]) { pq.prefetch = hw.out_w; pq.prefetch_bytes = DD; }
-            if (pf_force || !sh->sk[1]) { po.prefetch = hw.fc1_w; po.prefetch_bytes = 4 * DD; }
-            if (pf_force || !sh->sk[2]) { p1.prefetch = hw.fc2_w; p1.prefetch_bytes = 4 * DD; }
-            if ((pf_force || !sh->sk[3]) && i + 1 < nh) { p2.prefetch = h->halves[i + 1].qkv_w; p2.prefetch_bytes = 3 * DD; }
-        }
+        if (!sh->sk[0]) { pq.prefetch = hw.out_w; pq.prefetch_bytes = DD; }
+        if (!sh->sk[1]) { po.prefetch = hw.fc1_w; po.prefetch_bytes = 4 * DD; }
+        if (!sh->sk[2]) { p1.prefetch = hw.fc2_w; p1.prefetch_bytes = 4 * DD; }
+        if (!sh->sk[3] && i + 1 < nh) { p2.prefetch = h->halves[i + 1].qkv_w; p2.prefetch_bytes = 3 * DD; }
         // fused reduces: LN2 of this half after to_out, LN1 of the next half (or the final layer's norm) after fc2,
         // temporal attention after the temporal half's to_qkv
         SkinnyFuseParams f_out{}, f_fc2{}, f_qkv{};
@@ -190,13 +182,13 @@ int build_shape(gtav_dit_plan_s* p, Shape* sh, int frames, bool allow_skinny) {
         float* ws4[4];
         for (int k = 0; k < 4; ++k) ws4[k] = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(p->sk_ws) + k * p->sk_ws_bytes);
         const int tag = tag_enabled() ? (2 | ((i & 1) ^ 1)) : 0;
-        if (sh->sk[0]) { rc |= skinny_prepare(&sh->s_qkv[i], p->hn, D, static_cast<const bf16*>(hw.qkv_w), D, pq, EPI_STORE, ws4[0], p->sk_counters, so[0], ta ? &f_qkv : nullptr); sh->s_qkv[i].tag = tag; }
+        if (sh->sk[0]) { rc |= skinny_prepare(&sh->s_qkv[i], p->hn, D, static_cast<const bf16*>(hw.qkv_w), D, pq, EPI_STORE, ws4[0], p->sk_counters, 0, ta ? &f_qkv : nullptr); sh->s_qkv[i].tag = tag; }
         else rc |= gemm_prepare(&sh->g_qkv[i], p->hn, D, static_cast<const bf16*>(hw.qkv_w), D, pq, EPI_STORE);
-        if (sh->sk[1]) { rc |= skinny_prepare(&sh->s_out[i], p->att, D, static_cast<const bf16*>(hw.out_w), D, po, EPI_BIAS_GATE_RES, ws4[1], p->sk_counters, so[1], sh->fuse_ln ? &f_out : nullptr); sh->s_out[i].tag = tag; }
+        if (sh->sk[1]) { rc |= skinny_prepare(&sh->s_out[i], p->att, D, static_cast<const bf16*>(hw.out_w), D, po, EPI_BIAS_GATE_RES, ws4[1], p->sk_counters, 0, sh->fuse_ln ? &f_out : nullptr); sh->s_out[i].tag = tag; }
         else rc |= gemm_prepare(&sh->g_out[i], p->att, D, static_cast<const bf16*>(hw.out_w), D, po, EPI_BIAS_GATE_RES);
-        if (sh->sk[2]) { rc |= skinny_prepare(&sh->s_fc1[i], p->hn, D, static_cast<const bf16*>(hw.fc1_w), D, p1, EPI_BIAS_GELU_TANH, ws4[2], p->sk_counters, so[2]); sh->s_fc1[i].tag = tag; }
+        if (sh->sk[2]) { rc |= skinny_prepare(&sh->s_fc1[i], p->hn, D, static_cast<const bf16*>(hw.fc1_w), D, p1, EPI_BIAS_GELU_TANH, ws4[2], p->sk_counters); sh->s_fc1[i].tag = tag; }
         else rc |= gemm_prepare(&sh->g_fc1[i], p->hn, D, static_cast<const bf16*>(hw.fc1_w), D, p1, EPI_BIAS_GELU_TANH);
-        if (sh->sk[3]) { rc |= skinny_prepare(&sh->s_fc2[i], p->mlp, 4 * D, static_cast<const bf16*>(hw.fc2_w), 4 * D, p2, EPI_BIAS_GATE_RES, ws4[3], p->sk_counters, so[3], sh->fuse_ln ? &f_fc2 : nullptr); sh->s_fc2[i].tag = tag; }
+        if (sh->sk[3]) { rc |= skinny_prepare(&sh->s_fc2[i], p->mlp, 4 * D, static_cast<const bf16*>(hw.fc2_w), 4 * D, p2, EPI_BIAS_GATE_RES, ws4[3], p->sk_counters, 0, sh->fuse_ln ? &f_fc2 : nullptr); sh->s_fc2[i].tag = tag; }
         else rc |= gemm_prepare(&sh->g_fc2[i], p->mlp, 4 * D, static_cast<const bf16*>(hw.fc2_w), 4 * D, p2, EPI_BIAS_GATE_RES);
     }
     rc |= gemm_prepare(&sh->g_final, p->hn, D, static_cast<const bf16*>(w.final_w), D, gp(p->yfin, 64, w.final_b, M, h->out_feat, D), EPI_BIAS);

@@ -25,8 +25,7 @@
 //     the row-wise kernel that would follow - LayerNorm + modulate, or the last-frame temporal attention - run inside
 //     it; everything those need besides the partial sums is loaded BEFORE the partial sums.
 // Warp roles (256 threads): 0 = W producer, 1 = A producer, 2 = TMEM allocator + MMA issue (warp-uniform loop, elect.sync); all 8 warps drain the
-// accumulator (one TMEM lane quadrant each, half of the columns) and reduce.  (An optional L2 prefetch of the next GEMM's
-// weights, issued once the accumulator is complete, is off by default: GemmParams::prefetch, see dit_engine.cu.)
+// accumulator (one TMEM lane quadrant each, half of the columns) and reduce.
 #include "attn_temporal_core.cuh"
 #include "common.cuh"
 #include "kernels.h"
@@ -56,22 +55,14 @@ struct SkinnyParams {
 // Tagged partial sums: the exchange without fence, counter and poll.  The producer clears the lowest mantissa bit of every
 // fp32 partial sum and writes the launch's parity there; the consumer loads straight away and accepts an element once it
 // carries that parity, re-loading the ones that do not yet - every 4-byte element is its own ready flag, so no ordering
-// between elements is needed (relaxed gpu-scope stores and loads, L2 is the meeting point).  Stale elements always carry the
-// other parity because the caller (dit_engine.cu) gives each GEMM kind its own workspace, zeroed once, and alternates the
-// parity along the launches that share it: 1, 0, 1, 0 ... with an even number per pass.  Against the rendezvous protocol this
+// between elements is needed (relaxed gpu-scope stores and loads, L2 is the meeting point; ld.global.cg in the retry loop
+// never sees the other CTAs' stores, DESIGN.md 5b).  Stale elements always carry the other parity because the caller
+// (dit_engine.cu) gives each GEMM kind its own workspace, zeroed once, and alternates the parity along the launches that
+// share it: 1, 0, 1, 0 ... with an even number per pass.  Against the rendezvous protocol this
 // removes the gpu-scope fence after the stores, the atomic arrival, the polling round trip and two CTA barriers from the
 // critical path of every launch.  The sums lose their last mantissa bit (2^-24 relative, far below the bf16 rounding of the
 // Linear's output) and stay deterministic: summed in split order as before.  chk = 0: untagged, every element is accepted.
-#ifndef GTAV_SK_TAG_DELAY
-#define GTAV_SK_TAG_DELAY 600                      // SM clocks between a warp's last partial store and its first reduce load
-#endif
-#ifdef GTAV_SK_WEAK                                // A/B: the former .cg accesses instead of relaxed gpu-scope ones
-#define SK_LD "ld.global.cg"
-#define SK_ST "st.global.cg"
-#else
-#define SK_LD "ld.relaxed.gpu.global"
-#define SK_ST "st.relaxed.gpu.global"
-#endif
+static constexpr int SK_TAG_DELAY = 600;           // SM clocks between a warp's last partial store and its first reduce load
 struct SkTag {
     uint32_t chk, par;
 };
@@ -82,21 +73,21 @@ __device__ __forceinline__ bool tag_ok(uint4 v, SkTag t) {
 }
 __device__ __forceinline__ uint32_t ld_relaxed_u1(const float* p) {
     uint32_t v;
-    asm volatile(SK_LD ".u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
     return v;
 }
 __device__ __forceinline__ uint2 ld_relaxed_u2(const float* p) {
     uint2 v;
-    asm volatile(SK_LD ".v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p) : "memory");
+    asm volatile("ld.relaxed.gpu.global.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p) : "memory");
     return v;
 }
 __device__ __forceinline__ uint4 ld_relaxed_u4(const float* p) {
     uint4 v;
-    asm volatile(SK_LD ".v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
+    asm volatile("ld.relaxed.gpu.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
     return v;
 }
 __device__ __forceinline__ void st_relaxed_u1(float* p, uint32_t v) {
-    asm volatile(SK_ST ".u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+    asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 __device__ __forceinline__ void tag_spin_check(uint32_t& spins) {
     if (++spins > (1u << 21)) __trap();          // a protocol bug (parity out of step) fails the launch instead of hanging
@@ -618,11 +609,6 @@ gemm_skinny_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
         mbar_wait(bar_acc, 0);
         tcgen05_fence_after();
         if (threadIdx.x == 128) SK_STAMP(4);                                   // accumulator complete
-        // Optional (GTAV_PREFETCH=1; null by default): this CTA's operand slab has been consumed and HBM is idle for the
-        // rest of the launch (partials, rendezvous and reduce only move data through L2), so the NEXT GEMM's weights can be
-        // pulled into L2 here.  Measured: 1.191 vs 1.169 ms per last-frame step - the next launch's weight slab is not what
-        // its critical path waits for (its token slab lands at the same time); issued at kernel start (round 1) it cost 1.5 %.
-        l2_prefetch_share(p.g.prefetch, p.g.prefetch_bytes, blockIdx.x * SK_THREADS + threadIdx.x, p.gemm_ctas * SK_THREADS);
         const int c0 = warp < 4 ? half : 0;
         const uint32_t tlane = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + c0;
         float* mine = p.ws + static_cast<size_t>(blockIdx.x) * total * 128 + static_cast<size_t>(c0) * 128 + row;
@@ -640,11 +626,7 @@ gemm_skinny_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
         }
         if (!tagged) {
             // release: partial stores ordered before the arrival below - CTA barrier, then ONE gpu-scope fence by the arriving
-            // thread (cumulative over the barrier, the grid-sync idiom), then the relaxed atomic.  GTAV_SK_FENCE_ALL: every
-            // thread fences before the barrier instead (the former arrangement), kept for A/B measurement.
-#ifdef GTAV_SK_FENCE_ALL
-            asm volatile("fence.acq_rel.gpu;" ::: "memory");
-#endif
+            // thread (cumulative over the barrier, the grid-sync idiom), then the relaxed atomic.
             tcgen05_fence_before();
             __syncthreads();
             if (warp == 2) {                           // the accumulator has been read by everyone: give the TMEM back now,
@@ -652,9 +634,7 @@ gemm_skinny_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
                 tmem_dealloc(tmem_base, tmem_cols);
             }
             if (threadIdx.x == 128) {
-#ifndef GTAV_SK_FENCE_ALL
                 asm volatile("fence.acq_rel.gpu;" ::: "memory");
-#endif
                 SK_STAMP(5);                                                       // partials written + fenced
                 skinny_rendezvous(meet, meet_n, sense0);
             }
@@ -673,9 +653,7 @@ gemm_skinny_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
             } else {
                 asm volatile("bar.arrive 1, 256;" ::: "memory");
             }
-            if (GTAV_SK_TAG_DELAY > 0) {
-                while (clock64() - t0 < GTAV_SK_TAG_DELAY) {}
-            }
+            while (clock64() - t0 < SK_TAG_DELAY) {}
             if (threadIdx.x == 128) SK_STAMP(6);
         }
     } else if (FUSE != SK_FUSE_NONE && !tagged && threadIdx.x == 128) {

@@ -418,14 +418,9 @@ static int launch_one(const GemmOp* op, cudaStream_t stream) {
     // a single-round GEMM's epilogue is fully exposed, and the GELU one is the longest (measured in the real steps,
     // scripts/bench_step_b8.py: B = 8 last-frame step 2.645 -> 2.505 ms, dense B = 1 step 2.275 -> 2.119 ms).  4 warps (288
     // threads) for the other single-round GEMMs, where the extra warps only cost (gated-residual epilogue with 8: 2.84 ms;
-    // plain store: no change).  GTAV_EPI_WARPS=4|8 forces one value everywhere.
-    static int forced = -1;
-    if (forced < 0) {
-        const char* e = getenv("GTAV_EPI_WARPS");
-        forced = e == nullptr ? 0 : (e[0] == '4' ? 4 : 8);
-    }
+    // plain store: no change).
     const bool gelu = EPI == EPI_BIAS_GELU_TANH || EPI == EPI_BIAS_GELU_ERF;
-    const int epi_warps = forced ? forced : ((tiles > num_sms() || gelu) ? 8 : 4);
+    const int epi_warps = (tiles > num_sms() || gelu) ? 8 : 4;
     GTAV_CUDA_OK(launch_k(kern, grid, dim3(epi_warps == 8 ? GEMM_THREADS : 288), L::TOTAL, stream, op->tmA, op->tmB, op->p));
     return 0;
 }

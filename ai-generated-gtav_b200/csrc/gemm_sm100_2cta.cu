@@ -28,12 +28,8 @@ namespace gtav {
 static constexpr int G2_BM = 128;              // rows per CTA (256 per pair)
 static constexpr int G2_BN = 256;
 static constexpr int G2_BK = 64;
-#ifndef GTAV_G2_KC                             // (overridable for A/B builds: scripts/ab_define.sh)
-#define GTAV_G2_KC 2
-#define GTAV_G2_STAGES 3
-#endif
-static constexpr int G2_KC = GTAV_G2_KC;       // 64-wide K chunks per stage
-static constexpr int G2_STAGES = GTAV_G2_STAGES;
+static constexpr int G2_KC = 2;                // 64-wide K chunks per stage
+static constexpr int G2_STAGES = 3;
 static constexpr int G2_THREADS = 416;             // 13 warps: 5 producer / MMA + 8 epilogue
 static constexpr int G2_A_CHUNK = G2_BM * G2_BK * 2;           // 16 KB
 static constexpr int G2_B_CHUNK = (G2_BN / 2) * G2_BK * 2;     // 16 KB: this CTA's half of the weight rows

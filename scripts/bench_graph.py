@@ -124,12 +124,9 @@ def engine_steps():
     rows = torch.arange(5, dtype=torch.int32, device=dev)
     out = torch.empty((1, 1, 16, 18, 32), dtype=torch.bfloat16, device=dev)
     for label, env in (("default (weight-streaming GEMM, LN + temporal attention in the reduce)", {}),
-                       ("next weights prefetched into L2 after the weight-streaming GEMM's MMAs", {"GTAV_PREFETCH": "1"}),
                        ("separate LN / temporal-attention kernels", {"GTAV_FUSE": "0"}),
-                       ("to_out with 16 K-splits", {"GTAV_SK_SPLITS": "0,16,0,0"}),
-                       ("tiled GEMM everywhere", {"GTAV_SKINNY": "0"}),
-                       ("no PDL", {"GTAV_PDL_OFF_NOTE": "set GTAV_PDL=0 before start to test"})):
-        if "GTAV_PDL_OFF_NOTE" in env or (env and "--default-only" in sys.argv):
+                       ("tiled GEMM everywhere", {"GTAV_SKINNY": "0"})):
+        if env and "--default-only" in sys.argv:
             continue
         for k, v in env.items():
             os.environ[k] = v
