@@ -7,7 +7,8 @@
 // This is 1.2 % (DiT) / 8.5 % (VAE) of the step's FLOPs, so round 1 keeps it on warp-level
 // mma.sync m16n8k16 tiles (flash-style: scores stay in registers, online softmax across key
 // blocks, P rounded to bf16 before P@V like the reference's fused SDPA backends).  q/k are rotated
-// in fp32 and rounded to bf16 once, as apply_rotary_emb does (rotary_embedding_torch.py:46-73).
+// as apply_rotary_emb does (rotary_embedding_torch.py:46-73): two fp32 products and their fp32 sum,
+// each rounded to nearest (no FMA contraction), then one rounding to bf16.
 #include <stdlib.h>
 
 #include "attn_seq.cuh"

@@ -20,10 +20,13 @@ __device__ __forceinline__ void ldmatrix_x4_trans(uint32_t (&r)[4], const void* 
                  : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
                  : "r"(smem_u32(smem_ptr)));
 }
-// rotate the adjacent pair packed in `u` by (cos, sin) and re-round to bf16
+// rotate the adjacent pair packed in `u` by (cos, sin) and re-round to bf16.  Both products and the sum are rounded
+// explicitly: the reference's t * cos + rotate_half(t) * sin rounds each of them (rotary_embedding_torch.py:46-73), and
+// an FMA contraction of one product into the sum moves an occasional element by a bf16 ulp.
 __device__ __forceinline__ uint32_t rotate_pair(uint32_t u, float2 cs) {
     const float2 x = unpack_bf16x2(u);
-    return pack_bf16x2(x.x * cs.x - x.y * cs.y, x.y * cs.x + x.x * cs.y);
+    return pack_bf16x2(__fsub_rn(__fmul_rn(x.x, cs.x), __fmul_rn(x.y, cs.y)),
+                       __fadd_rn(__fmul_rn(x.y, cs.x), __fmul_rn(x.x, cs.y)));
 }
 
 

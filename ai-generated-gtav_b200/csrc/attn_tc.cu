@@ -6,8 +6,8 @@
 // (reference model/vae.py:78-107: S = 576, rotary on head dims 0..31 only).  Head dim 64; one CTA per (sequence, head).
 //
 //   * K and V of the whole head are brought ONCE into shared memory with cp.async (all copies of a thread in flight
-//     together) as 128-byte-swizzled rows of 64 bf16; K is then rotated in place (fp32 math, one bf16 rounding -
-//     apply_rotary_emb, rotary_embedding_torch.py:46-73).  K is the K-major B operand of S = Q K^T, the same kind of
+//     together) as 128-byte-swizzled rows of 64 bf16; K is then rotated in place (rounded fp32 products and sum, then
+//     bf16 - apply_rotary_emb, rotary_embedding_torch.py:46-73).  K is the K-major B operand of S = Q K^T, the same kind of
 //     image of V is the MN-major B operand of O = P V (no transpose anywhere);
 //   * queries are processed in tiles of 128 rows (UMMA M = 128), staged the same way by two loader warps into a
 //     double-buffered slot while the previous tile is being worked on;
@@ -93,10 +93,12 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc, int
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(src_bytes) : "memory");
 }
 
-// rotate the adjacent pair packed in `u` by (cos, sin) and re-round to bf16 (fp32 math, one rounding)
+// rotate the adjacent pair packed in `u` by (cos, sin) and re-round to bf16: two rounded fp32 products, a rounded fp32
+// sum, then the bf16 rounding, as the reference's t * cos + rotate_half(t) * sin (no FMA contraction)
 __device__ __forceinline__ uint32_t rot_pair(uint32_t u, float2 cs) {
     const float2 x = unpack_bf16x2(u);
-    return pack_bf16x2(x.x * cs.x - x.y * cs.y, x.y * cs.x + x.x * cs.y);
+    return pack_bf16x2(__fsub_rn(__fmul_rn(x.x, cs.x), __fmul_rn(x.y, cs.y)),
+                       __fadd_rn(__fmul_rn(x.y, cs.x), __fmul_rn(x.x, cs.y)));
 }
 // byte offset of chunk c of row r inside a [rows][128 B] image with the 128-byte swizzle (chunk index ^ row % 8)
 __device__ __forceinline__ uint32_t sw128(int r, int c) { return static_cast<uint32_t>(r) * AT_ROWB + ((c ^ (r & 7)) << 4); }
