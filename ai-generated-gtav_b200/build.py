@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libgtav_b200.so")
-SOURCES = ["gemm_sm100.cu", "gemm_sm100_2cta.cu", "gemm_sm100_splitk.cu", "gemm_skinny.cu", "norm_mod.cu", "attn_mma.cu", "attn_tc.cu", "attn_temporal.cu", "elementwise.cu", "dit_engine.cu",
+SOURCES = ["gemm_sm100.cu", "gemm_sm100_2cta.cu", "gemm_sm100_splitk.cu", "gemm_skinny.cu", "norm_mod.cu", "attn_mma.cu", "attn_tc.cu", "attn_temporal.cu", "attn_temporal_long.cu", "elementwise.cu", "dit_engine.cu",
            "vae_engine.cu", "sampler.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--cudart", "shared",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-Xptxas", "-v"]

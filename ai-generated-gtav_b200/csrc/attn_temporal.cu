@@ -1,11 +1,12 @@
-// Causal attention over the (<= 8) frames of the sliding window, one problem per (rollout, spatial
+// Causal attention over the (<= 8) frames of a short sliding window, one problem per (rollout, spatial
 // position, head), with the 1-D rotary embedding on the frame index fused.
 //
 // Replaces TemporalAxialAttention's rearrange + rotate_queries_or_keys + causal SDPA (reference
 // model/attention.py:52-66; rotary_embedding_torch.py:186-209: positions are window-relative
 // arange(T), theta 1e4).  T x T scores with T <= 5 are far too small for tensor cores: this kernel
 // is L2/HBM-bound (reads the 3*D-wide qkv rows once, writes D), one warp per problem, each lane owns
-// one rotary pair (2 of the 64 head dims), dot products reduced with shuffles.
+// one rotary pair (2 of the 64 head dims), dot products reduced with shuffles.  Windows of 9..32 frames
+// (8..31 cached) run the kernels of attn_temporal_long.cu, which the launchers below dispatch to.
 #include "attn_temporal_core.cuh"
 #include "common.cuh"
 #include "kernels.h"
@@ -124,9 +125,8 @@ int launch_attention_temporal_last(const bf16* qkv, bf16* out, int B, int ctx_fr
         break;
     switch (ctx_frames) {
         GTAV_TL(0) GTAV_TL(1) GTAV_TL(2) GTAV_TL(3) GTAV_TL(4) GTAV_TL(5) GTAV_TL(6) GTAV_TL(7)
-        default:
-            set_error("temporal attention (last frame): %d cached frames unsupported (0..7)", ctx_frames);
-            return -1;
+        default:   // 8..31 cached frames (attn_temporal_long.cu); refuses anything else
+            return launch_attention_temporal_last_long(qkv, out, B, ctx_frames, positions, heads, rot, kv_cache, s);
     }
 #undef GTAV_TL
     return 0;
@@ -144,9 +144,8 @@ int launch_attention_temporal(const bf16* qkv, bf16* out, int B, int T, int posi
         break;
     switch (T) {
         GTAV_TA(1) GTAV_TA(2) GTAV_TA(3) GTAV_TA(4) GTAV_TA(5) GTAV_TA(6) GTAV_TA(7) GTAV_TA(8)
-        default:
-            set_error("temporal attention: window of %d frames unsupported (1..8)", T);
-            return -1;
+        default:   // 9..32 frames (attn_temporal_long.cu); refuses anything else
+            return launch_attention_temporal_long(qkv, out, B, T, positions, heads, rot, kv_cache, s);
     }
 #undef GTAV_TA
     return 0;

@@ -80,6 +80,8 @@ void carve(gtav_dit_plan_s* p, void* ws, size_t* total) {
     p->h1 = c.take(R * D);
     p->cact = c.take(R * D);
     p->mod = c.take(R * static_cast<size_t>(e->mod_width));
+    // every size in size_t: at 32 frames the K/V caches alone are depth * B * 31 * 144 * 2048 bf16 (2.3 GB for the
+    // 16-block DiT at B = 8), past what an int counts in elements
     const size_t ctx_rows = static_cast<size_t>(p->B) * (p->T - 1) * e->tokens;
     p->kv_cache = c.take(static_cast<size_t>(e->cfg.depth) * ctx_rows * 2 * D);
     const int m_last = p->B * e->tokens;
@@ -279,9 +281,9 @@ int gtav_abi_version(void) { return 5; }
 int gtav_dit_create(const gtav_dit_config* cfg, const gtav_dit_weights* w, gtav_dit_t* out) {
     if (!cfg || !w || !out) { set_error("dit_create: null argument"); return -1; }
     if (cfg->hidden != 1024 || cfg->heads != 16 || cfg->grid_h * cfg->grid_w != 144 ||
-        cfg->in_channels * cfg->patch * cfg->patch != 64 || cfg->depth < 1 || cfg->max_frames < 1 || cfg->max_frames > 8) {
+        cfg->in_channels * cfg->patch * cfg->patch != 64 || cfg->depth < 1 || cfg->max_frames < 1 || cfg->max_frames > 32) {
         set_error("dit_create: unsupported geometry (hidden=%d heads=%d grid=%dx%d patch=%d C=%d depth=%d max_frames=%d); "
-                  "kernels are built for hidden 1024, 16 heads of 64, 144 tokens, 64 patch features",
+                  "kernels are built for hidden 1024, 16 heads of 64, 144 tokens, 64 patch features, windows of 1..32 frames",
                   cfg->hidden, cfg->heads, cfg->grid_h, cfg->grid_w, cfg->patch, cfg->in_channels, cfg->depth, cfg->max_frames);
         return -1;
     }

@@ -162,6 +162,11 @@ int launch_attention_temporal(const bf16* qkv, bf16* out, int B, int T, int posi
 // rows [B*positions, ...], the context frames' K/V come from kv_cache [B*ctx_frames*positions, 2*H*64].
 int launch_attention_temporal_last(const bf16* qkv, bf16* out, int B, int ctx_frames, int positions, int heads,
                                    const float2* rot, const bf16* kv_cache, cudaStream_t s);
+// Long windows (attn_temporal_long.cu), reached through the two launchers above: T = 9..32, ctx_frames = 8..31.
+int launch_attention_temporal_long(const bf16* qkv, bf16* out, int B, int T, int positions, int heads, const float2* rot,
+                                   bf16* kv_cache, cudaStream_t s);
+int launch_attention_temporal_last_long(const bf16* qkv, bf16* out, int B, int ctx_frames, int positions, int heads,
+                                        const float2* rot, const bf16* kv_cache, cudaStream_t s);
 
 // ---------------------------------------------------------------- conditioning / patches / sampler (elementwise.cu)
 // temb[r, 0:128] = cos(t_r f), temb[r,128:256] = sin(t_r f) (bf16); aemb[r,:] = bf16(act_r @ Wa^T + ba) if actions.

@@ -21,7 +21,8 @@ What differs, all additive or documented in DESIGN.md:
     prompt is the dummy dataset's 5-frame blue->red clip (dummy_dataset.py:16-28), or --prompt_video x.pt;
   * torchvision.io.write_video no longer exists: the writer is cv2.VideoWriter (mp4v), or a .npy / .pt dump
     when --output_path ends in .npy / .pt;
-  * additive flags: --rollouts, --seed, --random_init, --timing_json, --stepwise, --prompt_video.
+  * additive flags: --rollouts, --seed, --random_init, --timing_json, --stepwise, --prompt_video, --max_frames
+    (sliding-window length, default 5 as generate.py:139 sets it; 1..32).
 """
 from __future__ import annotations
 
@@ -68,6 +69,8 @@ def build_parser() -> argparse.ArgumentParser:
                    help=".pt tensor [n>=4, 3, 360, 640] in [0,1] used as the prompt instead of the dummy clip")
     p.add_argument("--stepwise", action="store_true",
                    help="run the literal per-step Python loop of the reference through the drop-in modules")
+    p.add_argument("--max_frames", type=int, default=5,
+                   help="frames in the sliding window the DiT sees, 1..32 (reference: 5, generate.py:139)")
     p.add_argument("--timing_json", type=str, default=None, help="write a timing report to this path")
     return p
 
@@ -168,7 +171,7 @@ def main(argv=None):
     B = max(1, args.rollouts)
     total_frames = args.total_frames
     noise_abs_max, stabilization_level = 20, 15
-    model.max_frames = 5
+    model.max_frames = args.max_frames
     video, n_prompt = load_prompt(args, device)
     video = video.expand(B, *video.shape[1:]).contiguous()
     print(f"We will generate {total_frames} frames, starting with {n_prompt} frames.")

@@ -24,6 +24,15 @@ except ImportError:  # imported as top-level `model.dit` with the package direct
     import _native as N
 
 
+MAX_FRAMES = 32      # longest sliding window the temporal attention kernels run (csrc/attn_temporal_long.cu)
+
+
+def _check_max_frames(max_frames):
+    if not 1 <= max_frames <= MAX_FRAMES:
+        raise RuntimeError(f"gtav_b200.DiT: max_frames={max_frames} is unsupported: the temporal attention kernels run "
+                           f"sliding windows of 1 to {MAX_FRAMES} frames")
+
+
 class _Rotary(nn.Module):
     """Holds the `freqs` parameter of the reference's RotaryEmbedding so checkpoints load unchanged
     (model/rotary_embedding_torch.py:118-136); the angle tables are built in DiT._pack."""
@@ -45,6 +54,7 @@ class DiT(nn.Module):
     def __init__(self, input_h=18, input_w=32, patch_size=2, in_channels=16, hidden_size=1024, depth=12, num_heads=16,
                  mlp_ratio=4.0, external_cond_dim=25, max_frames=5):
         super().__init__()
+        _check_max_frames(max_frames)
         self.in_channels = in_channels
         self.out_channels = in_channels
         self.patch_size = patch_size
@@ -90,6 +100,7 @@ class DiT(nn.Module):
 
         self._engine = None      # (handle, keep-alive tensors)
         self._packed_sig = None
+        self._packed_max_frames = None
         self._plans = {}
         self._dirty = False
         self._pack_generation = 0
@@ -159,8 +170,12 @@ class DiT(nn.Module):
         adaLN linears are concatenated into one [depth*2*6D + 2D, D] matrix so that all modulation
         vectors come out of a single GEMM."""
         sig = self._signature()
-        if self._engine is not None and sig == self._packed_sig and not self._dirty:
+        # max_frames is a plain attribute the reference's generate.py sets after construction; the engine and its
+        # temporal rotary table are built for the value at packing time, so a new value re-packs like a weight change
+        if self._engine is not None and sig == self._packed_sig and self.max_frames == self._packed_max_frames \
+                and not self._dirty:
             return
+        _check_max_frames(self.max_frames)
         self._release()
         self._dirty = False
         self._pack_generation += 1
@@ -226,6 +241,7 @@ class DiT(nn.Module):
         N.check(lib.gtav_dit_create(C.byref(cfg), C.byref(w), C.byref(handle)), "gtav_dit_create")
         self._engine = (handle, keep)
         self._packed_sig = sig
+        self._packed_max_frames = self.max_frames
 
     def _plan(self, B, T, cond_rows=None):
         cond_rows = B * T if cond_rows is None else cond_rows

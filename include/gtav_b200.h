@@ -105,12 +105,15 @@ int gtav_ln_affine(const void* x, void* out, int M, int D, const float* w, const
  * qkv [groups*seq, 3*heads*64], out [groups*seq, heads*64], rot = (cos,sin) float pairs [seq][rot_pairs]. */
 int gtav_attention_seq(const void* qkv, void* out, int groups, int seq, int heads, const float* rot, int rot_pairs,
                        gtav_stream_t stream);
-/* Causal attention over frames with fused rotary (attention.py:41-66); rows ordered (b, t, position). */
+/* Causal attention over T = 1..32 frames with fused rotary (attention.py:41-66); rows ordered (b, t, position);
+ * rot = (cos,sin) [>= T][32].  Any other T is refused before a launch. */
 int gtav_attention_temporal(const void* qkv, void* out, int B, int T, int positions, int heads, const float* rot,
                             gtav_stream_t stream);
 /* The last frame of that attention only, against cached context K/V: qkv / out hold the last-frame rows
  * [B*positions, ...]; kv_cache [B*ctx_frames*positions, 2*heads*64] = (rotated K | V) of window frames
- * 0..ctx_frames-1, rows ordered (b, t, position); the query sits at window position ctx_frames. */
+ * 0..ctx_frames-1, rows ordered (b, t, position); the query sits at window position ctx_frames.  ctx_frames = 0..31
+ * (rot rows >= ctx_frames + 1); any other count is refused before a launch.  Same bits as row ctx_frames of
+ * gtav_attention_temporal over ctx_frames + 1 frames. */
 int gtav_attention_temporal_last(const void* qkv, void* out, int B, int ctx_frames, int positions, int heads,
                                  const float* rot, const void* kv_cache, gtav_stream_t stream);
 /* DDIM update of train_dit.py:110-123 over F frames of n elements. */
@@ -128,7 +131,7 @@ typedef struct {
     int patch;        /* 2 */
     int in_channels;  /* 16 */
     int act_dim;      /* external_cond_dim: 25, or 0 */
-    int max_frames;   /* rows in rot_temporal */
+    int max_frames;   /* sliding-window length, 1..32: rows in rot_temporal */
 } gtav_dit_config;
 
 typedef struct {
@@ -147,7 +150,7 @@ typedef struct {
     const void *final_w, *final_b;   /* [p*p*C, D],[p*p*C] final_layer.linear */
     const float* temb_freqs;         /* [128] exp(-ln(1e4) i/128) (dit.py:107-111) */
     const float* rot_spatial;        /* (cos,sin) [grid_h*grid_w][32] axial "pixel" angles (rotary...:290-317) */
-    const float* rot_temporal;       /* (cos,sin) [max_frames][32] (rotary...:186-209) */
+    const float* rot_temporal;       /* (cos,sin) [max_frames][32], max_frames <= 32 rows (rotary...:186-209) */
     const gtav_dit_half* halves;     /* [2*depth]: block0.s, block0.t, block1.s, ... */
 } gtav_dit_weights;
 
