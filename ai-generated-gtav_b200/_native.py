@@ -21,7 +21,8 @@ EXPORTS = [
     "gtav_dit_conditioning", "gtav_dit_backbone", "gtav_dit_forward", "gtav_vae_create", "gtav_vae_destroy",
     "gtav_vae_workspace_bytes", "gtav_vae_plan_create", "gtav_vae_plan_destroy", "gtav_vae_encode", "gtav_vae_encode_moments", "gtav_vae_decode",
     "gtav_sampler_cond_rows", "gtav_sampler_scratch_bytes", "gtav_sampler_create", "gtav_sampler_destroy",
-    "gtav_sampler_run_frame", "gtav_noise_clamp",
+    "gtav_sampler_run_frame", "gtav_noise_clamp", "gtav_attention_temporal_ragged", "gtav_attention_temporal_last_ragged",
+    "gtav_dit_plan_set_window_lengths",
 ]
 
 SAMPLER_GRAPH, SAMPLER_FRAME_CACHE = 1, 2      # gtav_sampler_flags
@@ -91,6 +92,9 @@ def load() -> C.CDLL:
         "gtav_attention_seq": [vp, vp, i, i, i, fp, i, vp],
         "gtav_attention_temporal": [vp, vp, i, i, i, i, fp, vp],
         "gtav_attention_temporal_last": [vp, vp, i, i, i, i, fp, vp, vp],
+        "gtav_attention_temporal_ragged": [vp, vp, i, i, i, i, fp, ip, vp, vp],
+        "gtav_attention_temporal_last_ragged": [vp, vp, i, i, i, i, fp, ip, vp, vp],
+        "gtav_dit_plan_set_window_lengths": [vp, ip],
         "gtav_ddim_update": [fp, vp, fp, i, i, fp, fp, ip, vp],
         "gtav_dit_create": [C.POINTER(DitConfig), C.POINTER(DitWeights), C.POINTER(vp)],
         "gtav_dit_destroy": [vp],

@@ -5,8 +5,14 @@
 // reduce (gemm_skinny.cu), so both produce the same bits from the same q / k / v.
 #pragma once
 #include "common.cuh"
+#include "kernels.h"
 
 namespace gtav {
+
+// Valid frames of rollout b in a ragged pass over `frames` slots (kernels.h, TemporalLens); warp-uniform.
+__device__ __forceinline__ int ragged_valid(const TemporalLens& r, int b, int frames) {
+    return min(max(r.len[b], r.lo), frames + r.sub) - r.sub;
+}
 
 // Every fp32 operation below is an explicit round-to-nearest intrinsic: the same source compiled into different kernels
 // must not be contracted into FMAs differently (the fused and the stand-alone paths are tested for equal bits), and

@@ -22,10 +22,13 @@ static constexpr int TL_MAX_FRAMES = 32;   // dense window
 static constexpr int TL_KEY_CHUNK = 8;     // keys whose warp reductions are issued back to back
 
 // qkv [B*T*P, 3D] rows (b, t, pos), out [B*T*P, D], rot float2 [T][32], kv_cache (optional) [B*T*P, 2D].
-template <int TMAX>
+// RAGGED: as attn_temporal_kernel<T, true> (attn_temporal.cu) - slots before the rollout's trailing valid frames are
+// padding (output and cache rows 0), valid slot t sits at rotary position t - off and attends to valid keys only, with the
+// arithmetic and order of row t - off of an (T - off)-frame window.
+template <int TMAX, bool RAGGED = false>
 __global__ void __launch_bounds__(TLD_WARPS * 32)
 attn_temporal_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int B, int T, int P, int heads,
-                          const float2* __restrict__ rot, bf16* __restrict__ kv_cache) {
+                          const float2* __restrict__ rot, bf16* __restrict__ kv_cache, TemporalLens lens) {
     __shared__ uint32_t sk[TLD_WARPS][TMAX][32], sv[TLD_WARPS][TMAX][32];
     pdl_trigger();
     pdl_wait();
@@ -41,6 +44,7 @@ attn_temporal_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, 
     const size_t frame_ld = static_cast<size_t>(P) * ld;
     uint32_t (&kc)[TMAX][32] = sk[warp];
     uint32_t (&vc)[TMAX][32] = sv[warp];
+    const int off = RAGGED ? T - ragged_valid(lens, b, T) : 0;      // padded slots of this rollout
 
     // rotated K and V of every frame, packed bf16x2; the loads of a group of frames are issued before their first use
     constexpr int G = 8;
@@ -59,29 +63,37 @@ attn_temporal_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, 
             }
 #pragma unroll
             for (int t = t0; t < t0 + G; ++t) {
-                const float2 k = rotary_pair_rn(unpack_bf16x2(ku[t - t0]), rot[(t < T ? t : 0) * 32 + lane]);
+                const float2 k = rotary_pair_rn(unpack_bf16x2(ku[t - t0]), rot[(t < T && t >= off ? t - off : 0) * 32 + lane]);
                 kc[t][lane] = pack_bf16x2(k.x, k.y);          // exact: rotary_pair_rn rounded both halves to bf16
                 vc[t][lane] = vu[t - t0];
                 if (kv_cache != nullptr && t < T) {
                     const size_t row = (static_cast<size_t>(b) * T + t) * P + pos;
                     bf16* c = kv_cache + row * (2 * D) + head * 64 + 2 * lane;
-                    *reinterpret_cast<uint32_t*>(c) = kc[t][lane];
-                    *reinterpret_cast<uint32_t*>(c + D) = vu[t - t0];
+                    const bool pad = RAGGED && t < off;
+                    *reinterpret_cast<uint32_t*>(c) = pad ? 0u : kc[t][lane];
+                    *reinterpret_cast<uint32_t*>(c + D) = pad ? 0u : vu[t - t0];
                 }
             }
         }
     }
 
+    if (RAGGED) {
+        for (int i = 0; i < off; ++i) {
+            const size_t row = (static_cast<size_t>(b) * T + i) * P + pos;
+            *reinterpret_cast<uint32_t*>(out + row * D + head * 64 + 2 * lane) = 0u;
+        }
+    }
 #pragma unroll 1
-    for (int i = 0; i < T; ++i) {
-        const float2 q = rotary_pair_rn(unpack_bf16x2(*reinterpret_cast<const uint32_t*>(base + i * frame_ld)), rot[i * 32 + lane]);
+    for (int i = off; i < T; ++i) {
+        const float2 q = rotary_pair_rn(unpack_bf16x2(*reinterpret_cast<const uint32_t*>(base + i * frame_ld)), rot[(i - off) * 32 + lane]);
         // Scores of keys 0..i.  Keys go in chunks: the five butterfly steps of a chunk's dot products are issued key after
         // key within each step (as temporal_last_core does), and chunks past the query are skipped (warp-uniform).  Per
-        // key the additions are warp_sum's, in its order.  Keys i < j of a live chunk are computed and ignored.
+        // key the additions are warp_sum's, in its order.  Keys i < j (and padded keys j < off) of a live chunk are computed
+        // and ignored.
         float s[TMAX];
 #pragma unroll
         for (int c = 0; c < TMAX; c += TL_KEY_CHUNK) {
-            if (c <= i) {
+            if (c <= i && c + TL_KEY_CHUNK > off) {
 #pragma unroll
                 for (int j = c; j < c + TL_KEY_CHUNK; ++j) s[j] = dot_pair_rn(q, unpack_bf16x2(kc[j][lane]));
 #pragma unroll
@@ -94,14 +106,14 @@ attn_temporal_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, 
         float m = -INFINITY;
 #pragma unroll
         for (int j = 0; j < TMAX; ++j)
-            if (j <= i) {
+            if (j <= i && j >= off) {
                 s[j] = __fmul_rn(s[j], 0.125f);
                 m = fmaxf(m, s[j]);
             }
         float l = 0.f;
 #pragma unroll
         for (int j = 0; j < TMAX; ++j)
-            if (j <= i) {
+            if (j <= i && j >= off) {
                 s[j] = __expf(__fsub_rn(s[j], m));
                 l = __fadd_rn(l, s[j]);
             }
@@ -109,7 +121,7 @@ attn_temporal_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, 
         float2 acc = make_float2(0.f, 0.f);
 #pragma unroll
         for (int j = 0; j < TMAX; ++j)
-            if (j <= i) {
+            if (j <= i && j >= off) {
                 const float2 v = unpack_bf16x2(vc[j][lane]);
                 const float p = bf16_round(__fmul_rn(s[j], inv));   // probabilities enter P@V as bf16
                 acc.x = __fmaf_rn(p, v.x, acc.x);
@@ -121,11 +133,12 @@ attn_temporal_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, 
 }
 
 // Last frame against tc (run-time, <= TMAX) cached frames: attn_temporal_last_kernel with the cache length as an argument.
-// Same loads and the same temporal_last_core, so the same bits as row tc of the dense kernel.
-template <int TMAX>
+// Same loads and the same temporal_last_core, so the same bits as row tc of the dense kernel.  RAGGED: rollout b attends to
+// the trailing ragged_valid(lens, b, tc) of its tc cached slots, as attn_temporal_last_kernel<TC, true>.
+template <int TMAX, bool RAGGED = false>
 __global__ void __launch_bounds__(TL_WARPS * 32)
 attn_temporal_last_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int B, int tc, int P, int heads,
-                               const float2* __restrict__ rot, const bf16* __restrict__ kv_cache) {
+                               const float2* __restrict__ rot, const bf16* __restrict__ kv_cache, TemporalLens lens) {
     pdl_trigger();
     pdl_wait();
     const int lane = threadIdx.x & 31;
@@ -139,6 +152,11 @@ attn_temporal_last_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ 
     const size_t qrow = static_cast<size_t>(b) * P + pos;
     const bf16* base = qkv + qrow * (3 * D) + head * 64 + 2 * lane;
     const bf16* cache = kv_cache + (static_cast<size_t>(b) * tc * P + pos) * (2 * D) + head * 64 + 2 * lane;
+    if (RAGGED) {                           // the trailing n of the tc cached slots
+        const int n = ragged_valid(lens, b, tc);
+        cache += static_cast<size_t>(tc - n) * P * (2 * D);
+        tc = n;
+    }
     uint32_t kc[TMAX], vc[TMAX];
     temporal_cache_load(kc, vc, tc, cache, static_cast<size_t>(P) * 2 * D, D);
     const float2 qx = unpack_bf16x2(*reinterpret_cast<const uint32_t*>(base));
@@ -148,7 +166,7 @@ attn_temporal_last_long_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ 
 }
 
 int launch_attention_temporal_long(const bf16* qkv, bf16* out, int B, int T, int positions, int heads, const float2* rot,
-                                   bf16* kv_cache, cudaStream_t s) {
+                                   bf16* kv_cache, const TemporalLens* lens, cudaStream_t s) {
     if (T < 9 || T > TL_MAX_FRAMES) {
         set_error("temporal attention: window of %d frames unsupported (1..32)", T);
         return -1;
@@ -156,13 +174,18 @@ int launch_attention_temporal_long(const bf16* qkv, bf16* out, int B, int T, int
     const long problems = static_cast<long>(B) * positions * heads;
     if (problems <= 0) return 0;
     const int grid = static_cast<int>((problems + TLD_WARPS - 1) / TLD_WARPS);
+    if (lens != nullptr) {
+        GTAV_CUDA_OK(launch_k(attn_temporal_long_kernel<TL_MAX_FRAMES, true>, dim3(grid), dim3(TLD_WARPS * 32), 0, s, qkv, out, B,
+                              T, positions, heads, rot, kv_cache, *lens));
+        return 0;
+    }
     GTAV_CUDA_OK(launch_k(attn_temporal_long_kernel<TL_MAX_FRAMES>, dim3(grid), dim3(TLD_WARPS * 32), 0, s, qkv, out, B, T,
-                          positions, heads, rot, kv_cache));
+                          positions, heads, rot, kv_cache, TemporalLens{}));
     return 0;
 }
 
 int launch_attention_temporal_last_long(const bf16* qkv, bf16* out, int B, int ctx_frames, int positions, int heads,
-                                        const float2* rot, const bf16* kv_cache, cudaStream_t s) {
+                                        const float2* rot, const bf16* kv_cache, const TemporalLens* lens, cudaStream_t s) {
     if (ctx_frames < 8 || ctx_frames > TL_MAX_FRAMES - 1) {
         set_error("temporal attention (last frame): %d cached frames unsupported (0..31)", ctx_frames);
         return -1;
@@ -174,8 +197,13 @@ int launch_attention_temporal_last_long(const bf16* qkv, bf16* out, int B, int c
         return -1;
     }
     const int grid = static_cast<int>((problems + TL_WARPS - 1) / TL_WARPS);
+    if (lens != nullptr) {
+        GTAV_CUDA_OK(launch_k(attn_temporal_last_long_kernel<TL_MAX_FRAMES - 1, true>, dim3(grid), dim3(TL_WARPS * 32), 0, s, qkv,
+                              out, B, ctx_frames, positions, heads, rot, kv_cache, *lens));
+        return 0;
+    }
     GTAV_CUDA_OK(launch_k(attn_temporal_last_long_kernel<TL_MAX_FRAMES - 1>, dim3(grid), dim3(TL_WARPS * 32), 0, s, qkv, out,
-                          B, ctx_frames, positions, heads, rot, kv_cache));
+                          B, ctx_frames, positions, heads, rot, kv_cache, TemporalLens{}));
     return 0;
 }
 

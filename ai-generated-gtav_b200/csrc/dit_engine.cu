@@ -47,6 +47,7 @@ struct gtav_dit_plan_s {
     size_t sk_ws_bytes;      // kind (to_qkv, to_out, fc1, fc2), so that the tagged exchange sees only its own shape's data
     int* sk_counters;
     bool sk_out_of_step = false;   // a last-frame pass failed part-way: the tagged exchange's parities no longer line up
+    const int* lengths = nullptr;  // device int32 [B] window lengths 1..T (gtav_dit_plan_set_window_lengths), or none: all T
     GemmOp g_t0, g_t2, g_ada;
     Shape full, ctx, last;   // all T frames / the T-1 context frames / the last frame only
 };
@@ -141,7 +142,8 @@ int build_shape(gtav_dit_plan_s* p, Shape* sh, int frames, bool allow_skinny) {
     if (sh->sk[2]) sh->s_fc1.resize(nh);
     if (sh->sk[3]) sh->s_fc2.resize(nh);
     sh->fuse_ln = sh->sk[1] && sh->sk[3] && fuse_enabled();
-    sh->fuse_tattn = sh->sk[0] && fuse_enabled() && skinny_pick_splits(M, 3 * D, D) == 4 && p->T - 1 <= 7;
+    // the fused temporal attention reads every rollout's full cache: a plan with window lengths runs the ragged kernel
+    sh->fuse_tattn = sh->sk[0] && fuse_enabled() && skinny_pick_splits(M, 3 * D, D) == 4 && p->T - 1 <= 7 && p->lengths == nullptr;
     const size_t cache_layer = static_cast<size_t>(p->B) * (p->T - 1) * S * 2 * D;
     for (int i = 0; i < nh && rc == 0; ++i) {
         const gtav_dit_half& hw = h->halves[i];
@@ -238,7 +240,16 @@ int run_backbone(gtav_dit_plan_s* p, const Shape* sh, int mode, const void* x, i
             rc = launch_attention_seq(p->qkv, p->att, F, S, c.heads, rot_s, 32, stream);
         } else {
             bf16* cache = p->kv_cache + static_cast<size_t>(i >> 1) * cache_layer;
-            if (mode == MODE_LAST) rc = launch_attention_temporal_last(p->qkv, p->att, p->B, p->T - 1, S, c.heads, rot_t, cache, stream);
+            // window lengths, less the window frames that the kernel's slots do not cover (the last-frame kernel's slots are
+            // the T - 1 cached frames; the context pass covers T - 1 frames, a full pass all T)
+            const int slots = mode == MODE_LAST ? p->T - 1 : sh->frames;
+            const TemporalLens lens{p->lengths, 1, p->T - slots};
+            if (p->lengths != nullptr && mode == MODE_LAST)
+                rc = launch_attention_temporal_last_ragged(p->qkv, p->att, p->B, p->T - 1, S, c.heads, rot_t, cache, lens, stream);
+            else if (p->lengths != nullptr)
+                rc = launch_attention_temporal_ragged(p->qkv, p->att, p->B, sh->frames, S, c.heads, rot_t,
+                                                      mode == MODE_CONTEXT ? cache : nullptr, lens, stream);
+            else if (mode == MODE_LAST) rc = launch_attention_temporal_last(p->qkv, p->att, p->B, p->T - 1, S, c.heads, rot_t, cache, stream);
             else rc = launch_attention_temporal(p->qkv, p->att, p->B, sh->frames, S, c.heads, rot_t, mode == MODE_CONTEXT ? cache : nullptr, stream);
         }
         if (rc) return rc;
@@ -360,6 +371,22 @@ int gtav_dit_plan_create(gtav_dit_t h, int B, int T, int cond_rows, void* worksp
 }
 
 void gtav_dit_plan_destroy(gtav_dit_plan_t p) { delete p; }
+
+int gtav_dit_plan_set_window_lengths(gtav_dit_plan_t p, const int* lengths) {
+    if (!p) { set_error("dit_plan_set_window_lengths: null plan"); return -1; }
+    if ((p->lengths == nullptr) == (lengths == nullptr)) {
+        p->lengths = lengths;
+        return 0;
+    }
+    // attaching or detaching switches the fused temporal attention of the last-frame shape off or back on
+    const int* before = p->lengths;
+    p->lengths = lengths;
+    Shape last;
+    const int rc = build_shape(p, &last, 1, true);
+    if (rc) { p->lengths = before; return rc < 0 ? rc : -1; }
+    p->last = last;
+    return 0;
+}
 
 int gtav_dit_conditioning(gtav_dit_plan_t p, const int64_t* t, const float* actions, gtav_stream_t stream) {
     if (!p || !t) { set_error("dit_conditioning: null argument"); return -1; }
@@ -515,6 +542,18 @@ int gtav_attention_temporal_last(const void* qkv, void* out, int B, int ctx_fram
                                  const float* rot, const void* kv_cache, gtav_stream_t stream) {
     return launch_attention_temporal_last(static_cast<const bf16*>(qkv), static_cast<bf16*>(out), B, ctx_frames, positions,
                                           heads, reinterpret_cast<const float2*>(rot), static_cast<const bf16*>(kv_cache), stream);
+}
+int gtav_attention_temporal_ragged(const void* qkv, void* out, int B, int T, int positions, int heads, const float* rot,
+                                   const int* valid, void* kv_cache, gtav_stream_t stream) {
+    return launch_attention_temporal_ragged(static_cast<const bf16*>(qkv), static_cast<bf16*>(out), B, T, positions, heads,
+                                            reinterpret_cast<const float2*>(rot), static_cast<bf16*>(kv_cache),
+                                            TemporalLens{valid, 0, 0}, stream);
+}
+int gtav_attention_temporal_last_ragged(const void* qkv, void* out, int B, int ctx_frames, int positions, int heads,
+                                        const float* rot, const int* ctx_valid, const void* kv_cache, gtav_stream_t stream) {
+    return launch_attention_temporal_last_ragged(static_cast<const bf16*>(qkv), static_cast<bf16*>(out), B, ctx_frames,
+                                                 positions, heads, reinterpret_cast<const float2*>(rot),
+                                                 static_cast<const bf16*>(kv_cache), TemporalLens{ctx_valid, 0, 0}, stream);
 }
 int gtav_ddim_update(const float* x, const void* v_bf16, float* out, int F, int n, const float* abar_t,
                      const float* abar_next, const int* final_flag, gtav_stream_t stream) {

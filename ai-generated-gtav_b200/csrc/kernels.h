@@ -162,11 +162,29 @@ int launch_attention_temporal(const bf16* qkv, bf16* out, int B, int T, int posi
 // rows [B*positions, ...], the context frames' K/V come from kv_cache [B*ctx_frames*positions, 2*H*64].
 int launch_attention_temporal_last(const bf16* qkv, bf16* out, int B, int ctx_frames, int positions, int heads,
                                    const float2* rot, const bf16* kv_cache, cudaStream_t s);
-// Long windows (attn_temporal_long.cu), reached through the two launchers above: T = 9..32, ctx_frames = 8..31.
+// Ragged windows: rollout b of a pass over `frames` slots has valid frames only in its trailing slots, at rotary positions
+// 0, 1, ... from the first valid slot; the slots before are padding.  The count is read on the device at launch time:
+// valid(b) = min(max(len[b], lo), frames + sub) - sub, so a bad length gives wrong numbers, never an out-of-range access.
+// A DiT plan passes its window lengths with lo = 1 and sub = the window frames the pass does not cover (0 for a full
+// window, 1 for the context and last-frame passes); the stand-alone entry points pass per-rollout counts with lo = sub = 0.
+struct TemporalLens {
+    const int* len;   // device int32 [B]
+    int lo, sub;
+};
+// Long windows (attn_temporal_long.cu), reached through the launchers above and below: T = 9..32, ctx_frames = 8..31;
+// lens == nullptr: every window full.
 int launch_attention_temporal_long(const bf16* qkv, bf16* out, int B, int T, int positions, int heads, const float2* rot,
-                                   bf16* kv_cache, cudaStream_t s);
+                                   bf16* kv_cache, const TemporalLens* lens, cudaStream_t s);
 int launch_attention_temporal_last_long(const bf16* qkv, bf16* out, int B, int ctx_frames, int positions, int heads,
-                                        const float2* rot, const bf16* kv_cache, cudaStream_t s);
+                                        const float2* rot, const bf16* kv_cache, const TemporalLens* lens, cudaStream_t s);
+// launch_attention_temporal with rollout b's valid frames in its trailing valid(b) slots (attending to valid keys only,
+// rotated at rot[slot - first valid slot]); padded rows get output 0 and, with kv_cache, cache rows 0.  T = 1..32.
+int launch_attention_temporal_ragged(const bf16* qkv, bf16* out, int B, int T, int positions, int heads, const float2* rot,
+                                     bf16* kv_cache, TemporalLens lens, cudaStream_t s);
+// launch_attention_temporal_last against the trailing valid(b) of the ctx_frames cached slots of rollout b, the query at
+// rotary position valid(b).  ctx_frames = 0..31.
+int launch_attention_temporal_last_ragged(const bf16* qkv, bf16* out, int B, int ctx_frames, int positions, int heads,
+                                          const float2* rot, const bf16* kv_cache, TemporalLens lens, cudaStream_t s);
 
 // ---------------------------------------------------------------- conditioning / patches / sampler (elementwise.cu)
 // temb[r, 0:128] = cos(t_r f), temb[r,128:256] = sin(t_r f) (bf16); aemb[r,:] = bf16(act_r @ Wa^T + ba) if actions.

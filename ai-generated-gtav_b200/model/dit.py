@@ -243,9 +243,11 @@ class DiT(nn.Module):
         self._packed_sig = sig
         self._packed_max_frames = self.max_frames
 
-    def _plan(self, B, T, cond_rows=None):
+    def _plan(self, B, T, cond_rows=None, owner=None):
+        """The (B, T, cond_rows) plan, shared by every caller; owner: a key of the caller's own for a plan nobody else uses
+        (a StreamPool attaches window lengths to its plan)."""
         cond_rows = B * T if cond_rows is None else cond_rows
-        key = (B, T, cond_rows)
+        key = (B, T, cond_rows) if owner is None else (B, T, cond_rows, owner)
         if key not in self._plans:
             lib = N.load()
             handle = self._engine[0]
@@ -260,6 +262,16 @@ class DiT(nn.Module):
                         "gtav_dit_plan_create")
             self._plans[key] = (plan, ws)
         return self._plans[key][0]
+
+    def _drop_plans(self, owner):
+        """Release the plans created with this owner key (pending work on them drains first)."""
+        keys = [k for k in self._plans if len(k) == 4 and k[3] == owner]
+        if not keys:
+            return
+        torch.cuda.synchronize()
+        lib = N.load()
+        for k in keys:
+            lib.gtav_dit_plan_destroy(self._plans.pop(k)[0])
 
     # ------------------------------------------------------------------ forward
     @torch.no_grad()

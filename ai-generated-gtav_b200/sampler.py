@@ -63,11 +63,18 @@ class Sampler:
         # first: a load_state_dict / in-place weight change / .to() since the last call re-packs the weights, which
         # releases every plan and (through DiT._release -> _invalidate) every cached context of this sampler
         self.dit._pack()
-        if key in self._ctx:
-            return self._ctx[key]
+        if key not in self._ctx:
+            self._ctx[key] = self._new_context(B, T, dev)
+        return self._ctx[key]
+
+    def _new_context(self, B, T, dev, lengths=None, owner=None):
+        """Sampler handle and buffers over a (B, T) DiT plan.  lengths: device int32 [B] window lengths attached to the
+        plan of `owner`'s own (StreamPool), before the sampler handle captures anything."""
         lib = N.load()
         rows = lib.gtav_sampler_cond_rows(B, T, self.steps)
-        plan = self.dit._plan(B, T, rows)
+        plan = self.dit._plan(B, T, rows, owner=owner)
+        if lengths is not None:
+            N.check(lib.gtav_dit_plan_set_window_lengths(plan, lengths.data_ptr()), "gtav_dit_plan_set_window_lengths")
         n = self.frame_elems
         x_win = torch.zeros((B, T, n), dtype=torch.float32, device=dev)
         v_out = torch.zeros((B, T, n), dtype=torch.bfloat16, device=dev)
@@ -80,9 +87,7 @@ class Sampler:
         N.check(lib.gtav_sampler_create(plan, B, T, self.steps, n, x_win.data_ptr(), v_out.data_ptr(), abar.data_ptr(), levels,
                                         sbase, scratch.numel() - 256, flags, N.current_stream(), C.byref(h)),
                 "gtav_sampler_create")
-        ctx = dict(h=h, plan=plan, x_win=x_win, v_out=v_out, scratch=scratch, abar=abar, rows=rows)
-        self._ctx[key] = ctx
-        return ctx
+        return dict(h=h, plan=plan, x_win=x_win, v_out=v_out, scratch=scratch, abar=abar, rows=rows, lengths=lengths)
 
     def close(self):
         lib = N.load()
@@ -118,15 +123,17 @@ class Sampler:
         return t, torch.cat([a_ctx, a_last]).to(torch.float32).contiguous()
 
     # ------------------------------------------------------------------ one generated frame
-    def _denoise_frame(self, ctx_latents, chunk, act_win, stream, steps_limit=None):
+    def _denoise_frame(self, ctx_latents, chunk, act_win, stream, steps_limit=None, ctx=None):
         """ctx_latents [B, T-1, n] fp32 (the window's context frames), chunk [B, n] N(0,1) draws for the new frame,
         act_win [B, T, A] or None -> the new frame's latent [B, n] (a view of the window buffer: copy it before the
-        next call).  Enqueued on `stream`: clamp, conditioning table, context pass + (steps+1) DDIM steps."""
+        next call).  Enqueued on `stream`: clamp, conditioning table, context pass + (steps+1) DDIM steps.
+        ctx: a context of the caller's own (_new_context) instead of this sampler's (B, T) one."""
         lib = N.load()
         dev = chunk.device
         B, n = chunk.shape
         T = ctx_latents.shape[1] + 1
-        ctx = self._context(B, T, dev)
+        if ctx is None:
+            ctx = self._context(B, T, dev)
         xw = ctx["x_win"]
         xw[:, : T - 1] = ctx_latents
         N.check(lib.gtav_noise_clamp(chunk.data_ptr(), xw.data_ptr() + (T - 1) * n * 4, T * n, B, n,
@@ -211,6 +218,11 @@ class Sampler:
         FrameStream whose next(action) denoises ONE new frame against the sliding window and decodes only that frame."""
         return FrameStream(self, prompt_video, prompt_actions, generator)
 
+    def pool(self, capacity, use_actions=False):
+        """Interactive sessions that join and leave one batch: a StreamPool of `capacity` slots, each session a FrameStream
+        of B = 1 that runs batched with the others."""
+        return StreamPool(self, capacity, use_actions)
+
 
 class FrameStream:
     """Interactive rollout over a Sampler: the window of the last max_frames - 1 latents (and their actions) is kept on
@@ -270,3 +282,171 @@ class FrameStream:
         latent = new.reshape(B, *self.shape)
         frame = s.decode_frames(latent.unsqueeze(1))[:, 0] if decode else None
         return frame, latent
+
+
+class StreamPool:
+    """A fixed set of `capacity` slots, each holding one interactive session (a B = 1 FrameStream's state: the last
+    max_frames - 1 latents and actions on the device).  step() generates one frame for every open session in one batched
+    call: the pool's own (capacity, max_frames) DiT plan with per-slot window lengths attached
+    (gtav_dit_plan_set_window_lengths), so a session that joined recently runs its short, left-padded window next to full
+    ones.  Free slots run as length-1 windows and their results are dropped; the batch never changes shape, so one captured
+    frame graph serves every step.  Each session gets what a B = 1 FrameStream with the same prompt, actions and noise gives
+    (tests/test_stream_pool_gpu.py): bit for bit with the tiled GEMMs, and within the frame cache's bounds on the default
+    path, whose GEMM kernels depend on the row count."""
+
+    def __init__(self, sampler: Sampler, capacity: int, use_actions: bool = False):
+        capacity = int(capacity)
+        if capacity < 1:
+            raise RuntimeError(f"StreamPool: capacity must be at least 1, got {capacity}")
+        self.s = sampler
+        self.capacity = capacity
+        self.use_actions = bool(use_actions)
+        self.dev = sampler.dit.final_layer.linear.weight.device
+        self._slots = [None] * capacity         # session id per slot
+        self._sessions = {}                     # id -> dict(slot, window [k, n], actions [k, A] or None, generator, shape)
+        self._next_id = 0
+        self._ctx = None
+        sampler.dit._dependants.add(self)       # dropped with the DiT's plans when the weights are re-packed
+
+    # ------------------------------------------------------------------ sessions
+    @torch.no_grad()
+    def open(self, prompt_video, prompt_actions=None, generator=None):
+        """prompt_video [n, 3, H, W] in [0, 1] (n >= 1); prompt_actions [n, A], required iff the pool uses actions.
+        Returns the new session's id."""
+        N.require_cuda(prompt_video, "prompt_video")
+        s, vae = self.s, self.s.vae
+        want = (3, vae.input_height, vae.input_width)
+        if prompt_video.dim() != 4 or prompt_video.shape[0] < 1 or tuple(prompt_video.shape[1:]) != want:
+            raise RuntimeError(f"StreamPool.open: prompt_video must be [n >= 1, {want[0]}, {want[1]}, {want[2]}], "
+                               f"got {tuple(prompt_video.shape)}")
+        if (prompt_actions is None) == self.use_actions:
+            raise RuntimeError("StreamPool.open: pass prompt_actions iff the pool was created with use_actions=True")
+        if None not in self._slots:
+            raise RuntimeError(f"StreamPool.open: all {self.capacity} slots are taken")
+        n_prompt = prompt_video.shape[0]
+        keep = s.dit.max_frames - 1
+        actions = None
+        if prompt_actions is not None:
+            actions = prompt_actions.to(self.dev, torch.float32)
+            if tuple(actions.shape) != (n_prompt, s.dit.external_cond_dim):
+                raise RuntimeError(f"StreamPool.open: prompt_actions must be [n_prompt={n_prompt}, "
+                                   f"{s.dit.external_cond_dim}], got {tuple(prompt_actions.shape)}")
+            actions = actions[n_prompt - keep:] if keep > 0 else actions[:0]
+        lat = s.encode_prompt(prompt_video.to(self.dev)[None])[0]                 # [n, C, h, w]
+        window = lat.reshape(n_prompt, -1).float()
+        window = window[n_prompt - keep:] if keep > 0 else window[:0]
+        sid = self._next_id
+        self._next_id += 1
+        slot = self._slots.index(None)
+        self._slots[slot] = sid
+        self._sessions[sid] = dict(slot=slot, window=window.contiguous(), generator=generator, shape=tuple(lat.shape[1:]),
+                                   actions=None if actions is None else actions.contiguous())
+        return sid
+
+    def close(self, sid):
+        """Frees the session's slot for the next open()."""
+        self._session(sid, "close")
+        self._slots[self._sessions.pop(sid)["slot"]] = None
+
+    def _session(self, sid, what):
+        if sid not in self._sessions:
+            raise RuntimeError(f"StreamPool.{what}: no open session {sid!r}")
+        return self._sessions[sid]
+
+    @property
+    def sessions(self):
+        """Ids of the open sessions, in slot order."""
+        return [sid for sid in self._slots if sid is not None]
+
+    # ------------------------------------------------------------------ plan / sampler handle of the pool
+    def _context(self):
+        s = self.s
+        s.dit._pack()                           # a weight change releases the plans and (_invalidate) our handle
+        if self._ctx is None:
+            lengths = torch.ones(self.capacity, dtype=torch.int32, device=self.dev)
+            with torch.cuda.device(self.dev):
+                self._ctx = s._new_context(self.capacity, s.dit.max_frames, self.dev, lengths=lengths, owner=("pool", id(self)))
+        return self._ctx
+
+    def _release_context(self):
+        if self._ctx is not None:
+            torch.cuda.synchronize()
+            N.load().gtav_sampler_destroy(self._ctx["h"])
+            self._ctx = None
+
+    def _invalidate(self):
+        """Called by the DiT before it releases its plans: the sampler handle and its graph refer to the pool's plan."""
+        self._release_context()
+
+    def __del__(self):
+        try:
+            self._release_context()
+            self.s.dit._drop_plans(("pool", id(self)))
+        except Exception:
+            pass
+
+    # ------------------------------------------------------------------ one frame for every session
+    @torch.no_grad()
+    def step(self, actions=None, noise=None, decode=True):
+        """actions: {session id: [A]} for every open session iff the pool uses actions; noise: optional {session id:
+        [C, h, w]} N(0, 1) draws (a session without an entry draws from its own generator, as a B = 1 FrameStream).
+        Returns {session id: (uint8 frame [H, W, 3] or None, latent [C, h, w])}."""
+        s, dev, cap = self.s, self.dev, self.capacity
+        n = s.frame_elems
+        actions = {} if actions is None else dict(actions)
+        noise = {} if noise is None else dict(noise)
+        for sid in list(actions) + list(noise):
+            self._session(sid, "step")
+        open_ids = self.sessions
+        if not self.use_actions and actions:
+            raise RuntimeError("StreamPool.step: the pool was created without actions; pass none")
+        if self.use_actions and set(actions) != set(open_ids):
+            raise RuntimeError(f"StreamPool.step: an action is needed for every open session; missing "
+                               f"{sorted(set(open_ids) - set(actions))}")
+        if not open_ids:
+            return {}
+        ctx = self._context()
+        T = s.dit.max_frames
+        keep = T - 1
+        lens = [1] * cap
+        ctx_lat = torch.zeros((cap, T - 1, n), dtype=torch.float32, device=dev)      # left-padded windows
+        act_win = torch.zeros((cap, T, s.dit.external_cond_dim), dtype=torch.float32, device=dev) if self.use_actions else None
+        chunk = torch.zeros((cap, n), dtype=torch.float32, device=dev)
+        for sid in open_ids:
+            ses = self._sessions[sid]
+            b, k = ses["slot"], ses["window"].shape[0]
+            lens[b] = k + 1
+            if k:
+                ctx_lat[b, T - 1 - k:] = ses["window"]
+            if act_win is not None:
+                a = actions[sid].to(dev, torch.float32).reshape(-1)
+                if k:
+                    act_win[b, T - 1 - k: T - 1] = ses["actions"]
+                act_win[b, T - 1] = a
+            if sid in noise:
+                chunk[b] = noise[sid].to(device=dev, dtype=torch.float32).reshape(n)
+            else:
+                chunk[b] = torch.randn((1, n), device=dev, generator=ses["generator"])[0]
+        if s.use_graph and s._stream is None:
+            s._stream = torch.cuda.Stream(device=dev)
+        stream = s._stream if s.use_graph else torch.cuda.current_stream(dev)
+        stream.wait_stream(torch.cuda.current_stream(dev))
+        with torch.cuda.device(dev), torch.cuda.stream(stream):
+            # on the stream that replays the frame graph, so the graph reads this step's lengths
+            ctx["lengths"].copy_(torch.tensor(lens, dtype=torch.int32))
+            new = s._denoise_frame(ctx_lat, chunk, act_win, stream, ctx=ctx).clone()
+        torch.cuda.current_stream(dev).wait_stream(stream)
+        out = {}
+        for sid in open_ids:
+            ses = self._sessions[sid]
+            b = ses["slot"]
+            if keep > 0:
+                ses["window"] = torch.cat([ses["window"], new[b][None]])[-keep:].contiguous()
+                if act_win is not None:
+                    ses["actions"] = act_win[b, T - 1 - (lens[b] - 1):].clone()[-keep:].contiguous()
+            out[sid] = (None, new[b].reshape(ses["shape"]))
+        if decode:
+            lat = torch.stack([out[sid][1] for sid in open_ids])
+            frames = s.decode_frames(lat.unsqueeze(1))[:, 0]
+            out = {sid: (frames[i], out[sid][1]) for i, sid in enumerate(open_ids)}
+        return out

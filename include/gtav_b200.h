@@ -32,8 +32,9 @@ extern "C" {
 typedef struct CUstream_st* gtav_stream_t; /* == cudaStream_t */
 
 const char* gtav_last_error(void);
-/* ABI version; bumped on any signature change or new entry point (4: gtav_gemm_skinny_tagged_bf16, larger DiT plan workspace;
- * 5: gtav_gemm_skinny_fused_bf16). */
+/* ABI version; bumped on any change to an existing signature or behaviour (4: gtav_gemm_skinny_tagged_bf16, larger DiT plan
+ * workspace; 5: gtav_gemm_skinny_fused_bf16).  Purely additive entry points keep the version: 5 also has the ragged temporal
+ * attention (gtav_attention_temporal_ragged / _last_ragged) and gtav_dit_plan_set_window_lengths. */
 int gtav_abi_version(void);
 
 /* ------------------------------------------------------------------------------------------
@@ -116,6 +117,20 @@ int gtav_attention_temporal(const void* qkv, void* out, int B, int T, int positi
  * gtav_attention_temporal over ctx_frames + 1 frames. */
 int gtav_attention_temporal_last(const void* qkv, void* out, int B, int ctx_frames, int positions, int heads,
                                  const float* rot, const void* kv_cache, gtav_stream_t stream);
+/* Ragged windows of gtav_attention_temporal: valid int32 [B] on device, valid[b] in 0..T = the number of trailing valid
+ * frames of rollout b.  Its frames sit in slots T - valid[b] .. T - 1 at rotary positions 0 .. valid[b] - 1 and attend
+ * causally to valid frames only; each valid row gives the bits of gtav_attention_temporal run on that rollout's valid frames
+ * alone (T = valid[b]).  Padded rows get output 0.  kv_cache (NULL = none) [B*T*positions, 2*heads*64] receives the rotated
+ * K | V of valid rows and 0 in padded rows.  Values outside 0..T are clamped on the device.  A NULL valid and any T that
+ * gtav_attention_temporal refuses are refused before a launch. */
+int gtav_attention_temporal_ragged(const void* qkv, void* out, int B, int T, int positions, int heads, const float* rot,
+                                   const int* valid, void* kv_cache, gtav_stream_t stream);
+/* Ragged windows of gtav_attention_temporal_last: rollout b attends to the trailing ctx_valid[b] (0..ctx_frames, int32 [B] on
+ * device, clamped) of its ctx_frames cached frames, its query at rotary position ctx_valid[b] - the bits of
+ * gtav_attention_temporal_last at ctx_frames = ctx_valid[b] on those cache rows.  A NULL ctx_valid and any ctx_frames that
+ * gtav_attention_temporal_last refuses are refused before a launch. */
+int gtav_attention_temporal_last_ragged(const void* qkv, void* out, int B, int ctx_frames, int positions, int heads,
+                                        const float* rot, const int* ctx_valid, const void* kv_cache, gtav_stream_t stream);
 /* DDIM update of train_dit.py:110-123 over F frames of n elements. */
 int gtav_ddim_update(const float* x, const void* v_bf16, float* out, int F, int n, const float* abar_t,
                      const float* abar_next, const int* final_flag, gtav_stream_t stream);
@@ -171,6 +186,16 @@ size_t gtav_dit_workspace_bytes(gtav_dit_t h, int B, int T, int cond_rows);
 int gtav_dit_plan_create(gtav_dit_t h, int B, int T, int cond_rows, void* workspace, size_t workspace_bytes,
                          gtav_stream_t stream, gtav_dit_plan_t* out);
 void gtav_dit_plan_destroy(gtav_dit_plan_t p);
+/* Per-rollout window lengths: lengths int32 [B] on device, lengths[b] in 1..T.  Rollout b's window is left-padded: its
+ * frames sit in slots T - lengths[b] .. T - 1 at rotary positions 0 .. lengths[b] - 1, and the frame generated is slot T - 1.
+ * Every later gtav_dit_context / _last_frame / _backbone / _forward on the plan reads the lengths on the device when its
+ * kernels run (a captured graph reads the values current at replay), so they may change between passes.  The temporal
+ * attention then attends to valid frames only; padded frames are computed, never attended to, and their temporal attention
+ * output and cache rows are 0.  Each rollout's valid frames get what a plan of T = lengths[b] computes for that rollout alone.
+ * Lengths outside 1..T are clamped on the device (wrong numbers, never a fault).  A plan with lengths runs the temporal
+ * attention as a kernel of its own, not fused into the weight-streaming to_qkv GEMM (same bits).  NULL detaches the lengths.
+ * Attaching or detaching rebuilds the plan's launch descriptors: call it before gtav_sampler_create on the plan. */
+int gtav_dit_plan_set_window_lengths(gtav_dit_plan_t p, const int* lengths);
 
 /* Conditioning table: SiLU(t_embedder(t) + external_cond(a)) -> all adaLN modulation vectors
  * (dit.py:359-364 and the adaLN_modulation of 137-139,177-179,196-198) for cond_rows rows.
